@@ -1,6 +1,6 @@
 """bench.py — headline benchmark of the B200-native dquartic hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): default denoiser (1,204,738,391 parameters, dquartic_train_config.json),
 bf16 tensor-core mid stage / fp32 elsewhere, synthetic multiplexed MS2 maps of the config's shape
@@ -22,11 +22,25 @@ One JSON line on rank 0:
   strong     (N > 1) the same step at a GLOBAL batch of 256 (256 / N per GPU); dp_check: N-rank gradient vs one rank on
              the union batch
 `--impl reference` times the reference's own `_train_one_batch` (oracle/_ref) on the host cores, one sample per step.
+
+`--dump-outputs DIR` writes what the last timed step of `value` handed its caller, as float32 / float64 .npy files, so
+that two builds run with the same arguments (hence the same inputs) can be compared output for output (`bench_outputs/`
+at the repository root is git-ignored):
+  loss.npy               the mean loss `_train_one_batch` returned (float64 scalar)
+  x0.npy, ms2_cond.npy   the multiplexed batch, 2^20 fixed, seeded positions of each
+  ms1_cond.npy           the MS1 conditioning of the batch, whole
+  params.npy, grads.npy  the parameters after the optimizer step and the step's gradients: per parameter tensor, in
+                         state-dict order, all of it or 4096 fixed, seeded positions; the two arrays line up element
+                         for element, with zeros in grads.npy for tensors without a gradient (the rotary freqs).
+                         With N > 1 ranks they come from rank 0, and grads.npy is rank 0's gradient buffer after the
+                         exchange: under the sharded optimizer only the pieces rank 0 owns hold the reduced sum
 """
 import argparse
+import atexit
 import json
 import os
 import random
+import shutil
 import subprocess
 import sys
 import threading
@@ -235,6 +249,39 @@ def workload_config(world, micro_batch, per_gpu_batch):
     }
 
 
+DUMP_BATCH_ELEMS = 1 << 20
+DUMP_PER_TENSOR = 4096
+
+
+def _sample_positions(torch, np, rng, t, k):
+    """Index tuple of k seeded positions of `t` (sorted, drawn with replacement), or of every position if it has <= k."""
+    n = t.numel()
+    flat = np.arange(n) if n <= k else np.sort(rng.integers(0, n, size=k))
+    return tuple(torch.from_numpy(i).to(t.device) for i in np.unravel_index(flat, tuple(t.shape)))
+
+
+def dump_outputs(out_dir, torch, np, net, last):
+    """--dump-outputs: see the module docstring.  The positions come from one fixed seed and depend only on the shapes,
+    so every build of the same model samples the same elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(1234)
+    arrays = {"loss": np.float64(last["loss"])}
+    for name in ("x0", "ms2_cond"):
+        t = last[name]
+        arrays[name] = t[_sample_positions(torch, np, rng, t, DUMP_BATCH_ELEMS)].float().cpu().numpy()
+    arrays["ms1_cond"] = last["ms1_cond"].float().cpu().numpy()
+    net.sync_params()
+    ps, gs = [], []
+    for _, p in net.named_parameters():
+        idx = _sample_positions(torch, np, rng, p, DUMP_PER_TENSOR)
+        ps.append(p.detach()[idx].float().cpu())
+        gs.append(torch.zeros_like(ps[-1]) if p.grad is None else p.grad[idx].float().cpu())
+    arrays["params"] = torch.cat(ps).numpy()
+    arrays["grads"] = torch.cat(gs).numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- our arm
 def main():
     ap = argparse.ArgumentParser()
@@ -251,7 +298,12 @@ def main():
     ap.add_argument("--sample-chunk", type=int, default=64)
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as .npy files to DIR")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -287,6 +339,7 @@ def main():
     # ---- synthetic pool (same on every rank), written to npy so the public DIAMSDataset path is used
     import tempfile
     tmp = tempfile.mkdtemp(prefix=f"dq_bench_{rank}_")
+    atexit.register(shutil.rmtree, tmp, ignore_errors=True)   # 2.8 GB at the default pool; the dataset maps it until exit
     ms2, ms1 = synth_pool(args.pool, RT, MZ, seed=1234)
     np.save(os.path.join(tmp, "ms2.npy"), ms2)
     np.save(os.path.join(tmp, "ms1.npy"), ms1)
@@ -326,7 +379,9 @@ def main():
         return loader.draw(B)
 
     # ---- value: inputs resident in HBM when the timed region starts
-    def run_loop(n_warm, n_timed, e2e):
+    last = {}   # --dump-outputs: what the last timed step of `value` handed its caller
+
+    def run_loop(n_warm, n_timed, e2e, keep_last=False):
         loader = pin_loader if e2e else hbm_loader
         for i in range(n_warm):
             if e2e:
@@ -358,9 +413,11 @@ def main():
                 # pool resident in HBM: pair drawing (host, python `random` as in the reference), then ONE kernel chain
                 # gathers / normalises / mixes the 256 drawn pairs; all inside the timed region
                 x0, m1, other, m2, cond = loader.make_batch(draw(loader), want_cond=True)
-                ddim._train_one_batch(x0, cond, m1)
+                loss = ddim._train_one_batch(x0, cond, m1)
         ev1.record()
         barrier()
+        if keep_last:
+            last.update(loss=loss, x0=x0, ms2_cond=cond, ms1_cond=m1)
         ms = ev0.elapsed_time(ev1)
         if world > 1:
             t = torch.tensor([ms], device=dev)
@@ -371,8 +428,11 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_total, launches = run_loop(args.warmup, args.steps, e2e=False)
+    ms_total, launches = run_loop(args.warmup, args.steps, e2e=False, keep_last=bool(args.dump_outputs))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, np, net, last)
+    last.clear()
     ms_step = ms_total / args.steps
     value = B * world / (ms_step / 1000.0)
 

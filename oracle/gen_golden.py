@@ -8,6 +8,7 @@ the CUDA path (tests/test_*_gpu.py).  /root/reference does not exist on the GPU 
 smoke or bench time reads it.
 
     python oracle/gen_golden.py            # regenerates tests/golden/*.npz
+    DQUARTIC_REFERENCE=CHECKOUT python oracle/gen_golden.py   # from a checkout elsewhere (oracle/make_ref.py)
 """
 import json
 import os
@@ -21,6 +22,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, os.path.join(HERE, "_shims"))
 sys.path.insert(0, "/root/reference")
+if os.environ.get("DQUARTIC_REFERENCE"):
+    sys.path.insert(0, os.environ["DQUARTIC_REFERENCE"])
 sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.join(ROOT, "diffusion-deconvolution-dia-msms-data_b200", "dquartic", "utils"))
 
@@ -106,25 +109,8 @@ def gen_unet():
     time = torch.tensor([7, 801], dtype=torch.long)
     with torch.no_grad():
         out = torch.cat([m(x[i:i + 1], time[i:i + 1], ic[i:i + 1], ac[i:i + 1]) for i in range(b)], dim=0)
-    # also intermediate activations of sample 0 for per-layer parity
-    acts = {}
-    hooks = []
-
-    def mk(name):
-        def hook(mod, inp, o):
-            acts[name] = o.detach().clone().numpy()
-        return hook
-
-    for name in ("init_conv", "downs.0.0", "downs.0.2", "downs.0.3", "downs.3.2", "downs.6.3", "mid_block1",
-                 "mid_attn", "mid_block2", "ups.0.0", "ups.0.3", "ups.6.2", "final_res_block"):
-        mod = m.get_submodule(name)
-        hooks.append(mod.register_forward_hook(mk(name)))
-    with torch.no_grad():
-        m(x[0:1], time[0:1], ic[0:1], ac[0:1])
-    for h in hooks:
-        h.remove()
     np.savez_compressed(os.path.join(GOLD, "unet_tiny.npz"), x=x.numpy(), time=time.numpy(), init_cond=ic.numpy(),
-                        attn_cond=ac.numpy(), out=out.numpy(), **{"act:" + k: v for k, v in acts.items()})
+                        attn_cond=ac.numpy(), out=out.numpy())
     print("unet ok", out.shape, float(out.abs().mean()))
 
 
@@ -168,12 +154,12 @@ def gen_train():
     out = dict(x0=x0.numpy(), ms2_cond=c2.numpy(), ms1_cond=c1.numpy(), t=t.numpy(), noise=noise.numpy(),
                loss_per_sample=losses.numpy(), loss=np.float32(losses.mean().item()),
                total_norm=np.float32(total_norm.item()), lr=np.float32(lr))
-    for k, g in grads.items():
-        out["grad:" + k] = g.numpy()
     for k in ("init_conv.weight", "downs.0.0.block1.proj.weight", "mid_block1.block1.proj.weight",
               "mid_attn.fn.fn.to_qv.weight", "ups.6.2.fn.fn.to_out.1.g", "final_conv.bias", "time_mlp.1.weight"):
         out["new:" + k] = new[k].numpy()
     np.savez_compressed(os.path.join(GOLD, "train_tiny.npz"), **out)
+    # the gradients in a file of their own: one archive with everything would pass 1 MB
+    np.savez_compressed(os.path.join(GOLD, "train_tiny_grads.npz"), **{"grad:" + k: g.numpy() for k, g in grads.items()})
     print("train ok", losses, float(total_norm))
 
 

@@ -152,12 +152,24 @@ def test_lr_schedule_and_optimizer_state_format():
 
 
 def test_config_loader_override_rules(tmp_path):
+    """The generated default config against the reference's shipped dquartic_train_config.json, compared as loaded
+    dicts.  The original file is read from a reference checkout when one is present (oracle/make_ref.py: argument,
+    DQUARTIC_REFERENCE or the default location).  tests/golden/default_train_config.json is NOT that file's bytes: it
+    is this project's own generate_train_config() output at the time the test stopped depending on a checkout, kept so
+    that the default cannot drift where no checkout exists.  Four of its values are checked independently against
+    what SURVEY.md quotes from the shipped file."""
+    import make_ref
+
     p = str(tmp_path / "cfg.json")
     generate_train_config(p)
-    ref = json.load(open("/root/reference/dquartic_train_config.json")) if os.path.exists("/root/reference") else None
     cfg = load_train_config(p)
-    if ref is not None:
-        assert cfg == ref
+    snapshot = json.load(open(os.path.join(ROOT, "tests", "golden", "default_train_config.json")))
+    assert cfg == snapshot
+    assert snapshot["model"]["batch_size"] == 1 and snapshot["model"]["learning_rate"] == 1e-5
+    assert snapshot["model"]["ms1_loss_weight"] == 0.0 and snapshot["wandb"]["wandb_mode"] == "offline"
+    shipped = os.path.join(make_ref.checkout()[0], "dquartic_train_config.json")
+    if os.path.exists(shipped):
+        assert cfg == json.load(open(shipped))
     cfg = load_train_config(p, batch_size=8, checkpoint_path=None, use_wandb=False, threads=2, ms2_data_path="a.npy")
     assert cfg["model"]["batch_size"] == 8 and cfg["model"]["checkpoint_path"] == "best_model.ckpt"
     assert cfg["wandb"]["use_wandb"] is False and cfg["threads"] == 2 and cfg["data"]["ms2_data_path"] == "a.npy"

@@ -44,6 +44,7 @@ def test_train_step_loss_and_gradients_match_reference_golden():
     from dquartic.model.model import DDIMDiffusionModel
 
     g = golden("train_tiny.npz")
+    gg = golden("train_tiny_grads.npz")
     net, P = make_net()
     net.train()
     d = DDIMDiffusionModel(net, device="cuda")
@@ -59,7 +60,7 @@ def test_train_step_loss_and_gradients_match_reference_golden():
     for k in P:
         if k.endswith("freqs"):
             continue
-        ref = torch.from_numpy(g["grad:" + k])
+        ref = torch.from_numpy(gg["grad:" + k])
         got = net._params[k].grad
         e = rel_err(got, ref)
         worst = max(worst, e)

@@ -61,6 +61,7 @@ def test_unet_forward_matches_reference(golden_dir):
 
 def test_train_step_loss_and_grads_match_reference(golden_dir):
     g = _load(golden_dir, "train_tiny.npz")
+    gg = _load(golden_dir, "train_tiny_grads.npz")
     P = {k: v.clone().requires_grad_(not k.endswith("freqs")) for k, v in O.det_params(TINY).items()}
     _, _, ab = O.schedule_tables(1000, "cosine")
     loss, _ = O.train_loss(P, TINY, ab, torch.from_numpy(g["x0"]), torch.from_numpy(g["ms2_cond"]),
@@ -69,7 +70,7 @@ def test_train_step_loss_and_grads_match_reference(golden_dir):
     loss.backward()
     names = [k for k in P if P[k].requires_grad]
     for k in names:
-        ref = g["grad:" + k]
+        ref = gg["grad:" + k]
         got = P[k].grad.numpy()
         scale = max(np.abs(ref).max(), 1e-6)
         assert np.abs(got - ref).max() <= 2e-4 * scale + 1e-7, k
@@ -79,7 +80,7 @@ def test_train_step_loss_and_grads_match_reference(golden_dir):
     # optimizer arithmetic is checked on the REFERENCE's gradients so that the first-step sign(g)-like
     # update (m / (sqrt(v) + eps) with |g| ~ eps) is not sensitive to 1e-4-level gradient differences
     lr = float(g["lr"])
-    ref_grads = [torch.from_numpy(g["grad:" + k]) for k in names]
+    ref_grads = [torch.from_numpy(gg["grad:" + k]) for k in names]
     clipped, total = O.clip_grad_norm(ref_grads)
     assert abs(float(total) - float(g["total_norm"])) < 1e-5 * float(g["total_norm"])
     for k, gc in zip(names, clipped):

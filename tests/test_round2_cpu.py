@@ -157,15 +157,33 @@ def test_optimizer_shard_layout_covers_the_buffer_once():
     assert (cover == 1).all()
 
 
-def test_reference_vendoring_recipe_runs_where_the_reference_is():
+def test_reference_vendoring_recipe_runs_where_the_reference_is(tmp_path):
+    """oracle/make_ref.py on a stand-in checkout with the reference's layout: the hot-path modules are copied unmodified,
+    package markers and shims are added; without a checkout it is a no-op that succeeds (build() calls it that way)."""
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, os.path.join(root, "oracle", "make_ref.py")], capture_output=True, text=True)
+    script = os.path.join(root, "oracle", "make_ref.py")
+    env = {k: v for k, v in os.environ.items() if k != "DQUARTIC_REFERENCE"}
+    r = subprocess.run([sys.executable, script], capture_output=True, text=True, env=env)
     assert r.returncode == 0, r.stderr
-    if os.path.isdir("/root/reference/dquartic"):
-        for rel in ("dquartic/model/model.py", "dquartic/model/unet1d.py", "rotary_embedding_torch.py"):
-            assert os.path.exists(os.path.join(root, "oracle", "_ref", rel))
+    checkout, dst = tmp_path / "reference", tmp_path / "_ref"
+    rels = ("model/model.py", "model/model_interface.py", "model/unet1d.py", "model/building_blocks.py",
+            "utils/data_loader.py")
+    for rel in rels:
+        (checkout / "dquartic" / rel).parent.mkdir(parents=True, exist_ok=True)
+        (checkout / "dquartic" / rel).write_text(f"# {rel}\n")
+    r = subprocess.run([sys.executable, script, str(checkout), str(dst)], capture_output=True, text=True, env=env)
+    assert r.returncode == 0, r.stderr
+    for rel in rels:
+        assert (dst / "dquartic" / rel).read_text() == f"# {rel}\n"
+    for rel in ("dquartic/__init__.py", "dquartic/model/__init__.py", "dquartic/utils/__init__.py"):
+        assert (dst / rel).exists()
+    for shim in ("rotary_embedding_torch.py", "duckdb.py"):
+        assert (dst / shim).read_bytes() == open(os.path.join(root, "oracle", "_shims", shim), "rb").read()
+    r = subprocess.run([sys.executable, script, str(tmp_path / "missing"), str(dst)], capture_output=True, text=True,
+                       env=env)
+    assert r.returncode != 0
 
 
 def test_deferred_parameter_gathers_are_awaited_before_the_parameters_are_read():

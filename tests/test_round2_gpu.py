@@ -272,7 +272,7 @@ def test_sample_windows_is_independent_of_the_sharding_and_matches_sample():
 
 @pytest.mark.parametrize("C,L,pre", [(4, 4500, "downs.1.2"), (8, 1300, "downs.2.2"), (12, 2049, "downs.5.2"),
                                      (16, 700, "ups.0.2")])
-def test_tcgen05_linear_attention_backward_matches_mma_sync_kernel(C, L, pre):
+def test_tcgen05_linear_attention_backward_matches_mma_sync_kernel(C, L, pre, tmp_path):
     """The tcgen05 / TMEM backward (q path) against the mma.sync TF32 kernel it replaces, same inputs, and the pipeline
     must not have timed out (dq_la_tc_last_error)."""
     import subprocess
@@ -292,18 +292,19 @@ def test_tcgen05_linear_attention_backward_matches_mma_sync_kernel(C, L, pre):
     assert _native.la_tc_last_error() is None
     names = [k for k in net._params if k.startswith(pre + ".")]
     got = {k: net._params[k].grad.clone().cpu() for k in names}
-    torch.save({"x": x.cpu(), "dres": dres.cpu()}, "/tmp/_la_ab_in.pt")
+    f_in, f_out = str(tmp_path / "la_ab_in.pt"), str(tmp_path / "la_ab_out.pt")
+    torch.save({"x": x.cpu(), "dres": dres.cpu()}, f_in)
     code = (
         "import sys, torch\n"
         f"sys.path[:0] = {sys.path!r}\n"
         "from _util import make_net\n"
         "net, _ = make_net(seed=7); net._ensure_grads(); net._gflat.zero_()\n"
-        "d = torch.load('/tmp/_la_ab_in.pt')\n"
+        f"d = torch.load({f_in!r})\n"
         f"out, saved = net._la_fwd({pre!r}, d['x'].cuda(), True); dx = net._la_bwd({pre!r}, saved, d['dres'].cuda())\n"
-        f"torch.save({{'dx': dx.cpu(), **{{k: net._params[k].grad.cpu() for k in net._params if k.startswith({pre!r} + '.')}}}}, '/tmp/_la_ab_out.pt')\n")
+        f"torch.save({{'dx': dx.cpu(), **{{k: net._params[k].grad.cpu() for k in net._params if k.startswith({pre!r} + '.')}}}}, {f_out!r})\n")
     env = dict(os.environ, DQ_LA_TC="0")
     subprocess.run([sys.executable, "-c", code], check=True, env=env)
-    ref = torch.load("/tmp/_la_ab_out.pt")
+    ref = torch.load(f_out)
     assert rel_err(dx, ref["dx"]) < 5e-3
     for k in names:
         assert rel_err(got[k], ref[k]) < 5e-3, k

@@ -5,6 +5,7 @@ from _util import make_net, golden, rel_err
 from dquartic.model.model import DDIMDiffusionModel
 
 g = golden("train_tiny.npz")
+gg = golden("train_tiny_grads.npz")
 net, P = make_net()
 net.train()
 d = DDIMDiffusionModel(net, device="cuda")
@@ -17,7 +18,7 @@ print("loss", float(loss.mean()), float(g["loss"]))
 rows = []
 for k in P:
     if k.endswith("freqs"): continue
-    ref = torch.from_numpy(g["grad:" + k]); got = net._params[k].grad.cpu()
+    ref = torch.from_numpy(gg["grad:" + k]); got = net._params[k].grad.cpu()
     e = float((got - ref).abs().max() / ref.abs().max().clamp_min(1e-30))
     cos = float(torch.dot(got.flatten(), ref.flatten()) / (got.norm() * ref.norm()).clamp_min(1e-30))
     rows.append((e, cos, k, float(ref.abs().max())))
