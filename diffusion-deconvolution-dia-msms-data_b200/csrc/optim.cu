@@ -2,7 +2,8 @@
 // coefficient on the device (no host sync), AdamW with decoupled weight decay, and the bf16 (+ transposed)
 // operand refresh for the tcgen05 GEMMs (mid.cu: cast_transpose).
 // Replaces (reference /root/reference/dquartic/model/model_interface.py): clip_grad_norm_(max_norm=10) 1121,
-// torch.optim.AdamW(lr) 1011 / optimizer.step() 1122.  Traffic: 4 B/param (norm) + 28 B/param (update).
+// torch.optim.AdamW(lr) 1011 / optimizer.step() 1122.  Traffic: 4 B/param (norm) + 28 B/param (update; 36 B/param with
+// the weight EMA of dq_adamw_ema).
 #include "common.cuh"
 
 namespace dq {
@@ -55,10 +56,17 @@ __device__ __forceinline__ void adamw_update(float& pi, float gi, float& mi, flo
   pi = __fmaf_rn(-step_size, __fdiv_rn(mi, denom), pi);
 }
 
+// Exponential moving average of the updated weight, ema += (1 - beta) (p - ema), rounded like adamw_update.
+__device__ __forceinline__ void ema_update(float pi, float& ei, float ema_w) { ei = __fmaf_rn(__fsub_rn(pi, ei), ema_w, ei); }
+
+// kEma: the same pass also moves the EMA buffer `ema` towards the updated weights (dq_adamw_ema): one more 4-byte load
+// and store per element (36 instead of 28 B/param) instead of a second 12 B/param pass.
+template <bool kEma>
 __global__ void __launch_bounds__(256) adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
-                                                    float* __restrict__ m, float* __restrict__ v, long n,
-                                                    const float* __restrict__ coef_ptr, float lr, float b1, float b2,
-                                                    float eps, float wd, float step_size, float bc2_sqrt) {
+                                                    float* __restrict__ m, float* __restrict__ v, float* __restrict__ ema,
+                                                    long n, const float* __restrict__ coef_ptr, float lr, float b1,
+                                                    float b2, float eps, float wd, float step_size, float bc2_sqrt,
+                                                    float ema_w) {
   const float coef = coef_ptr ? coef_ptr[1] : 1.f;
   const long stride = (long)gridDim.x * blockDim.x;
   const float decay = 1.f - lr * wd;
@@ -66,16 +74,24 @@ __global__ void __launch_bounds__(256) adamw_kernel(float* __restrict__ p, const
     float pi = p[i], mi = m[i], vi = v[i];
     adamw_update(pi, g[i], mi, vi, coef, decay, b1, b2, eps, step_size, bc2_sqrt);
     p[i] = pi; m[i] = mi; v[i] = vi;
+    if constexpr (kEma) {
+      float ei = ema[i];
+      ema_update(pi, ei, ema_w);
+      ema[i] = ei;
+    }
   }
 }
 
-// The same update on 16-byte vectors (all four arrays 16-byte aligned: the whole flat buffer and the mid-stage ranges):
-// 4 x 16-byte loads + 3 x 16-byte stores per thread and iteration instead of 7 four-byte accesses; the n % 4 tail
-// elements are handled by the first threads of the grid.  Arithmetic identical to adamw_kernel, element by element.
+// The same update on 16-byte vectors (all arrays 16-byte aligned: the whole flat buffer and the mid-stage ranges):
+// 4 (5 with the EMA) x 16-byte loads + 3 (4) x 16-byte stores per thread and iteration instead of 7 (9) four-byte
+// accesses; the n % 4 tail elements are handled by the first threads of the grid.  Arithmetic identical to adamw_kernel,
+// element by element.
+template <bool kEma>
 __global__ void __launch_bounds__(256) adamw4_kernel(float* __restrict__ p, const float* __restrict__ g,
-                                                     float* __restrict__ m, float* __restrict__ v, long n,
-                                                     const float* __restrict__ coef_ptr, float lr, float b1, float b2,
-                                                     float eps, float wd, float step_size, float bc2_sqrt) {
+                                                     float* __restrict__ m, float* __restrict__ v, float* __restrict__ ema,
+                                                     long n, const float* __restrict__ coef_ptr, float lr, float b1,
+                                                     float b2, float eps, float wd, float step_size, float bc2_sqrt,
+                                                     float ema_w) {
   const float coef = coef_ptr ? coef_ptr[1] : 1.f;
   const long stride = (long)gridDim.x * blockDim.x;
   const float decay = 1.f - lr * wd;
@@ -93,6 +109,14 @@ __global__ void __launch_bounds__(256) adamw4_kernel(float* __restrict__ p, cons
     reinterpret_cast<float4*>(p)[i] = p4;
     reinterpret_cast<float4*>(m)[i] = m4;
     reinterpret_cast<float4*>(v)[i] = v4;
+    if constexpr (kEma) {
+      float4 e4 = reinterpret_cast<float4*>(ema)[i];
+      ema_update(p4.x, e4.x, ema_w);
+      ema_update(p4.y, e4.y, ema_w);
+      ema_update(p4.z, e4.z, ema_w);
+      ema_update(p4.w, e4.w, ema_w);
+      reinterpret_cast<float4*>(ema)[i] = e4;
+    }
   }
   const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (t < (n & 3)) {
@@ -100,6 +124,38 @@ __global__ void __launch_bounds__(256) adamw4_kernel(float* __restrict__ p, cons
     float pi = p[i], mi = m[i], vi = v[i];
     upd(pi, g[i], mi, vi);
     p[i] = pi; m[i] = mi; v[i] = vi;
+    if constexpr (kEma) {
+      float ei = ema[i];
+      ema_update(pi, ei, ema_w);
+      ema[i] = ei;
+    }
+  }
+}
+
+// Exchange two buffers in place (sampling from the EMA weights without a parameter-sized temporary).
+__global__ void __launch_bounds__(256) swap_kernel(float* __restrict__ a, float* __restrict__ b, long n) {
+  const long stride = (long)gridDim.x * blockDim.x;
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const float t = a[i];
+    a[i] = b[i];
+    b[i] = t;
+  }
+}
+
+__global__ void __launch_bounds__(256) swap4_kernel(float* __restrict__ a, float* __restrict__ b, long n) {
+  const long stride = (long)gridDim.x * blockDim.x;
+  const long n4 = n >> 2;
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    const float4 t = reinterpret_cast<float4*>(a)[i];
+    reinterpret_cast<float4*>(a)[i] = reinterpret_cast<float4*>(b)[i];
+    reinterpret_cast<float4*>(b)[i] = t;
+  }
+  const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < (n & 3)) {
+    const long i = (n4 << 2) + t;
+    const float x = a[i];
+    a[i] = b[i];
+    b[i] = x;
   }
 }
 
@@ -125,21 +181,46 @@ DQ_API int dq_clip_coef(const double* sumsq, float max_norm, float gscale, float
   DQ_LAUNCH_CHECK();
   return 0;
 }
-DQ_API int dq_adamw(float* p, const float* g, float* m, float* v, long n, const float* coef_ptr, float lr, float b1,
-                    float b2, float eps, float wd, float step_size, float bc2_sqrt, void* stream) {
-  if (n <= 0) return 0;
-  long b = (n + 256L * 8 - 1) / (256L * 8);
+// Grid of an elementwise kernel over n elements, `per_thread` of them per thread, at most 16 blocks per SM.
+static unsigned ew_blocks(long n, long per_thread) {
+  long b = (n + 256L * per_thread - 1) / (256L * per_thread);
   if (b > 148L * 16) b = 148L * 16;
   if (b < 1) b = 1;
-  if (((((size_t)p) | ((size_t)g) | ((size_t)m) | ((size_t)v)) & 15) == 0 && n >= 4) {
-    long b4 = (n / 4 + 256L * 4 - 1) / (256L * 4);
-    if (b4 > 148L * 16) b4 = 148L * 16;
-    if (b4 < 1) b4 = 1;
-    adamw4_kernel<<<(unsigned)b4, 256, 0, (cudaStream_t)stream>>>(p, g, m, v, n, coef_ptr, lr, b1, b2, eps, wd, step_size, bc2_sqrt);
+  return (unsigned)b;
+}
+
+template <bool kEma>
+static int launch_adamw(float* p, const float* g, float* m, float* v, float* ema, long n, const float* coef_ptr,
+                        float lr, float b1, float b2, float eps, float wd, float step_size, float bc2_sqrt, float ema_w,
+                        void* stream) {
+  if (n <= 0) return 0;
+  if (((((size_t)p) | ((size_t)g) | ((size_t)m) | ((size_t)v) | ((size_t)ema)) & 15) == 0 && n >= 4) {
+    adamw4_kernel<kEma><<<ew_blocks(n / 4, 4), 256, 0, (cudaStream_t)stream>>>(p, g, m, v, ema, n, coef_ptr, lr, b1, b2,
+                                                                               eps, wd, step_size, bc2_sqrt, ema_w);
     DQ_LAUNCH_CHECK();
     return 0;
   }
-  adamw_kernel<<<(unsigned)b, 256, 0, (cudaStream_t)stream>>>(p, g, m, v, n, coef_ptr, lr, b1, b2, eps, wd, step_size, bc2_sqrt);
+  adamw_kernel<kEma><<<ew_blocks(n, 8), 256, 0, (cudaStream_t)stream>>>(p, g, m, v, ema, n, coef_ptr, lr, b1, b2, eps, wd,
+                                                                        step_size, bc2_sqrt, ema_w);
+  DQ_LAUNCH_CHECK();
+  return 0;
+}
+
+DQ_API int dq_adamw(float* p, const float* g, float* m, float* v, long n, const float* coef_ptr, float lr, float b1,
+                    float b2, float eps, float wd, float step_size, float bc2_sqrt, void* stream) {
+  return launch_adamw<false>(p, g, m, v, nullptr, n, coef_ptr, lr, b1, b2, eps, wd, step_size, bc2_sqrt, 0.f, stream);
+}
+DQ_API int dq_adamw_ema(float* p, const float* g, float* m, float* v, float* ema, long n, const float* coef_ptr,
+                        float lr, float b1, float b2, float eps, float wd, float step_size, float bc2_sqrt, float ema_w,
+                        void* stream) {
+  return launch_adamw<true>(p, g, m, v, ema, n, coef_ptr, lr, b1, b2, eps, wd, step_size, bc2_sqrt, ema_w, stream);
+}
+DQ_API int dq_swap(float* a, float* b, long n, void* stream) {
+  if (n <= 0) return 0;
+  if (((((size_t)a) | ((size_t)b)) & 15) == 0 && n >= 4)
+    swap4_kernel<<<ew_blocks(n / 4, 4), 256, 0, (cudaStream_t)stream>>>(a, b, n);
+  else
+    swap_kernel<<<ew_blocks(n, 8), 256, 0, (cudaStream_t)stream>>>(a, b, n);
   DQ_LAUNCH_CHECK();
   return 0;
 }

@@ -61,6 +61,8 @@ _SIGS = {
     "dq_sumsq": ("plps", 1),
     "dq_clip_coef": ("pffps", 1),
     "dq_adamw": ("pppplpfffffffs", 1),
+    "dq_adamw_ema": ("ppppplpffffffffs", 1),
+    "dq_swap": ("ppls", 1),
     "dq_fill": ("pfls", 1),
     "dq_multiplex": ("ppippffpppppilis", 3),
 }

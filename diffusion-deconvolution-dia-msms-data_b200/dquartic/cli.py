@@ -1,6 +1,7 @@
 """`dquartic` command line — same commands and options as the reference (/root/reference/dquartic/cli.py:26-188):
 `dquartic train CONFIG [--parquet_directory --ms2-data-path --ms1-data-path --batch-size --checkpoint-path
---use-wandb --threads]`, `dquartic generate-config`.  Differences: `--batch-size/--threads` are cast to int (the
+--use-wandb --threads]`, `dquartic generate-config`.  `--ema-decay` (model.ema_decay in the config) keeps an exponential
+moving average of the weights in the checkpoints.  Differences: `--batch-size/--threads` are cast to int (the
 reference passes strings to DataLoader and fails, SURVEY.md §5); under torchrun (RANK/WORLD_SIZE in the
 environment) each rank binds one GPU, joins an NCCL process group and trains a batch shard;
 `generate-train-data` (offline ETL) is out of scope.
@@ -55,7 +56,11 @@ def _init_distributed():
 @click.option("--checkpoint-path", default=None, help="Path to save the best model, overrides config file")
 @click.option("--use-wandb", default=None, cls=PythonLiteralOption, help="Use wandb for logging, overrides config file")
 @click.option("--threads", default=None, help="Number of threads for data loading, overrides config file")
-def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_size, checkpoint_path, use_wandb, threads):
+@click.option("--ema-decay", default=None, type=click.FloatRange(0.0, 1.0, min_open=True, max_open=True),
+              help="Keep an exponential moving average of the weights with this decay (e.g. 0.9999) and save it in the "
+                   "checkpoints as ema_state_dict, overrides config file")
+def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_size, checkpoint_path, use_wandb, threads,
+          ema_decay):
     """
     Train a DDIM model on the DIAMS dataset.
     """
@@ -74,7 +79,7 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
 
     config = load_train_config(config_path, parquet_directory=parquet_directory, ms2_data_path=ms2_data_path,
                                ms1_data_path=ms1_data_path, batch_size=batch_size, checkpoint_path=checkpoint_path,
-                               use_wandb=use_wandb, threads=threads)
+                               use_wandb=use_wandb, threads=threads, ema_decay=ema_decay)
     batch_size = int(config["model"]["batch_size"])
     checkpoint_path = config["model"]["checkpoint_path"]
     use_wandb = config["wandb"]["use_wandb"]
@@ -115,6 +120,7 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
         auto_normalize=config["model"]["auto_normalize"], ms1_loss_weight=config["model"]["ms1_loss_weight"],
         device=device)
     diffusion_model.micro_batch = int(os.environ.get("DQUARTIC_MICRO_BATCH", "0")) or None
+    diffusion_model.ema_decay = config["model"].get("ema_decay")
 
     if use_wandb and rank == 0:
         import wandb

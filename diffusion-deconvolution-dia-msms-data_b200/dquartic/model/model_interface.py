@@ -6,7 +6,8 @@ grad-clip 10.0 + AdamW(lr, betas (0.9, 0.999), eps 1e-8, weight_decay 0.01), che
 (`epoch, model_state_dict, optimizer_state_dict, scheduler_state_dict, best_loss`) and file naming, the
 0.5/0.5 mixing of the two drawn samples, `predict` returning dicts `{ms2_1, ms1_1, mixture, pred}`.
 
-New: the optimizer step is three fused kernels over the flat parameter buffer (`FusedAdamW`); a batch larger than
+New: the optimizer step is three fused kernels over the flat parameter buffer (`FusedAdamW`), optionally keeping an
+exponential moving average of the weights in the same pass (`ema_decay`, `ema_weights()`); a batch larger than
 `micro_batch` is processed by gradient accumulation; under `torch.distributed` the batch is sharded by sample and
 the flat gradient is summed over the ranks in buckets (the four 300 M-parameter mid-block ranges are launched as soon as
 the mid-stage backward has produced them, overlapping the long down-path backward).  Those ranges (99 % of the
@@ -14,6 +15,7 @@ parameters) are REDUCE-SCATTERED: each rank keeps Adam moments for, and updates,
 pieces are all-gathered in place (ZeRO-1); 1 / world-size is folded into the clip coefficient; rank 0 writes checkpoints.
 Plotting / wandb tables (reference 669-976, 1152-1242) are out of scope (SURVEY.md §2).
 """
+import contextlib
 import functools
 import math
 import os
@@ -93,9 +95,16 @@ class FusedAdamW(torch.optim.Optimizer):
     coefficient (no averaging pass).  Sharded mode (`set_sharding`): the ranges listed there were reduce-scattered, this
     rank owns piece `rank` of each of them and keeps Adam moments for its pieces only (1 / world-size of the state,
     1 / world-size of the update traffic); the small rest of the buffer is replicated and updated by every rank; the
-    updated pieces are all-gathered in place into the flat parameter buffer."""
+    updated pieces are all-gathered in place into the flat parameter buffer.
 
-    def __init__(self, net, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2):
+    `ema_decay` (0 < ema_decay < 1, default None: off) keeps an exponential moving average of the weights, updated in
+    the same pass as AdamW (dq_adamw_ema) and laid out like the Adam moments (sharded mode: this rank's pieces plus the
+    replicated rest).  Update k (from 0) uses the decay min(ema_decay, (1 + k) / (10 + k)).  `swap_ema()` exchanges
+    it with the live weights; `ema_state_dict()` returns it in the model's state-dict format."""
+
+    def __init__(self, net, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, ema_decay=None):
+        if ema_decay is not None and not 0.0 < float(ema_decay) < 1.0:
+            raise ValueError(f"ema_decay must be None or in (0, 1), got {ema_decay}")
         self.net = net
         params = list(net.parameters())
         defaults = dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay, amsgrad=False, maximize=False,
@@ -109,6 +118,15 @@ class FusedAdamW(torch.optim.Optimizer):
         self._shard = None      # (rank, world, [(offset, numel)]) of the reduce-scattered ranges
         self._segments = None   # [(flat offset, numel, state offset)] this rank updates
         self._full_state = None
+        self.ema_decay = None if ema_decay is None else float(ema_decay)
+        self._ema = None            # EMA of the weights, same layout as _m / _v
+        self.ema_updates = 0        # EMA updates so far (k of the decay warm-up)
+        self._ema_swapped = False   # swap_ema(): the network holds the EMA, _ema the live weights
+
+    @staticmethod
+    def ema_beta(ema_decay, k):
+        """Decay of EMA update k (counting from 0): a short warm-up so that the average forgets the initial weights."""
+        return min(ema_decay, (1.0 + k) / (10.0 + k))
 
     # ---- layout of the state this rank keeps
     def set_sharding(self, rank, world, ranges):
@@ -142,6 +160,21 @@ class FusedAdamW(torch.optim.Optimizer):
             self._v = torch.zeros(total, dtype=torch.float32, device=flat.device)
             self._sumsq = torch.zeros(1, dtype=torch.float64, device=flat.device)
             self._coef = torch.zeros(2, dtype=torch.float32, device=flat.device)
+            if self.ema_decay is not None:
+                self._ema = torch.empty(total, dtype=torch.float32, device=flat.device)
+                self.reset_ema()
+
+    @torch.no_grad()
+    def reset_ema(self):
+        """Start the EMA over at the current weights (update count 0)."""
+        if self._ema_swapped:
+            raise RuntimeError("reset_ema() inside ema_weights()")
+        self._ensure_state()
+        flat = self.net.flat_params()
+        for (o, cnt, so) in self._segments:
+            self._ema[so:so + cnt].copy_(flat[o:o + cnt])
+        self.ema_updates = 0
+        self._full_state = None
 
     def zero_grad(self, set_to_none: bool = False):
         self.net.zero_grad()
@@ -150,6 +183,8 @@ class FusedAdamW(torch.optim.Optimizer):
     def step(self, closure=None, max_grad_norm=None, grad_scale=1.0, defer_gather=False):
         """`defer_gather` (sharded mode): leave the parameter all-gathers in flight on the NCCL stream; the network waits
         for them right before its mid stage (`UNet1d.sync_params`), so they overlap the next step's down path."""
+        if self._ema_swapped:
+            raise RuntimeError("FusedAdamW.step() while the network holds the EMA weights (inside ema_weights())")
         self._ensure_state()
         net = self.net
         g = net.flat_grads()
@@ -178,16 +213,19 @@ class FusedAdamW(torch.optim.Optimizer):
             self.last_grad_norm = self._coef[0:1]
         bc1 = 1.0 - b1 ** self._step
         bc2 = 1.0 - b2 ** self._step
+        ema = self._ema
+        if ema is not None:
+            ema_w = 1.0 - self.ema_beta(self.ema_decay, self.ema_updates)   # rounded to fp32 by the call
+            self.ema_updates += 1
         for (o, cnt, so) in self._segments:
-            N.call("dq_adamw", p[o:o + cnt], g[o:o + cnt], self._m[so:so + cnt], self._v[so:so + cnt], cnt, coef, lr, b1,
-                   b2, eps, wd, lr / bc1, math.sqrt(bc2))
+            if ema is None:
+                N.call("dq_adamw", p[o:o + cnt], g[o:o + cnt], self._m[so:so + cnt], self._v[so:so + cnt], cnt, coef, lr,
+                       b1, b2, eps, wd, lr / bc1, math.sqrt(bc2))
+            else:
+                N.call("dq_adamw_ema", p[o:o + cnt], g[o:o + cnt], self._m[so:so + cnt], self._v[so:so + cnt],
+                       ema[so:so + cnt], cnt, coef, lr, b1, b2, eps, wd, lr / bc1, math.sqrt(bc2), ema_w)
         if sharded:
-            rank, world, ranges = self._shard
-            works = []
-            for (o, cnt) in ranges:           # updated pieces -> every rank's flat parameter buffer, in place
-                k = cnt // world
-                works.append(torch.distributed.all_gather_into_tensor(p[o:o + cnt], p[o + rank * k:o + (rank + 1) * k],
-                                                                      async_op=True))
+            works = self._gather_params(p)
             if defer_gather and hasattr(net, "sync_params"):
                 net.__dict__.setdefault("_pending_param_works", []).extend(works)
             else:
@@ -196,28 +234,107 @@ class FusedAdamW(torch.optim.Optimizer):
         self._full_state = None
         net.mark_params_modified()
 
+    def _gather_params(self, p):
+        """Sharded mode: all-gather every rank's piece of the sharded ranges into the flat parameter buffer, in place."""
+        rank, world, ranges = self._shard
+        works = []
+        for (o, cnt) in ranges:
+            k = cnt // world
+            works.append(torch.distributed.all_gather_into_tensor(p[o:o + cnt], p[o + rank * k:o + (rank + 1) * k],
+                                                                  async_op=True))
+        return works
+
+    # ---- weight EMA ---------------------------------------------------------------------------------------
+    def _require_ema(self):
+        if self.ema_decay is None:
+            raise RuntimeError("this FusedAdamW keeps no weight EMA (ema_decay=None)")
+        self._ensure_state()
+
+    @torch.no_grad()
+    def swap_ema(self):
+        """Exchange the EMA and the live weights in the network's flat parameter buffer (sharded mode: a collective, every
+        rank; the swapped pieces are all-gathered).  Calling it twice restores the live weights bit for bit."""
+        self._require_ema()
+        net = self.net
+        p = net.flat_params()
+        for (o, cnt, so) in self._segments:
+            N.call("dq_swap", p[o:o + cnt], self._ema[so:so + cnt], cnt)
+        if self._shard is not None:
+            for w in self._gather_params(p):
+                w.wait()
+        self._ema_swapped = not self._ema_swapped
+        net.mark_params_modified()   # the bf16 GEMM operands are recast from the new weights
+
+    def _full_ema(self):
+        """EMA over the trainable flat range.  Sharded mode: needs `gather_state()` beforehand, unless the network holds
+        the EMA (swap_ema), whose buffer then has it in full on every rank."""
+        n = self.net.n_trainable_flat
+        if self._ema_swapped:
+            return self.net.flat_params()[:n]
+        if self._shard is None:
+            return self._ema
+        if self._full_state is None or len(self._full_state) < 3:
+            raise RuntimeError("sharded FusedAdamW: call gather_state() on every rank before ema_state_dict()")
+        return self._full_state[2]
+
+    @torch.no_grad()
+    def ema_state_dict(self, device=None):
+        """The EMA in the format of `UNet1d.state_dict()` (same names, shapes and order; the non-trainable rotary
+        frequencies are the live model's), as copies on `device` (default: the EMA's device)."""
+        self._require_ema()
+        net = self.net
+        full = self._full_ema()
+        out = {}
+        for name in net.state_dict(keep_vars=True):
+            par = net._params[name]
+            src = net._view(full, name) if par.requires_grad else par.detach()
+            dst = torch.empty(src.shape, dtype=src.dtype, device=src.device if device is None else device)
+            out[name] = dst.copy_(src)
+        return out
+
+    @torch.no_grad()
+    def load_ema_state_dict(self, sd, updates):
+        """Inverse of `ema_state_dict()`; `updates` is the EMA update count to resume from.  Sharded mode: this rank
+        keeps its own pieces and the replicated rest."""
+        self._require_ema()
+        if self._ema_swapped:
+            raise RuntimeError("load_ema_state_dict() inside ema_weights()")
+        net = self.net
+        if self._shard is None:
+            full = self._ema
+        else:
+            full = torch.zeros(net.n_trainable_flat, dtype=torch.float32, device=self._ema.device)
+        for name, par in net._params.items():
+            if par.requires_grad:
+                net._view(full, name).copy_(sd[name])
+        if self._shard is not None:
+            for (o, cnt, so) in self._segments:
+                self._ema[so:so + cnt].copy_(full[o:o + cnt])
+        self.ema_updates = int(updates)
+        self._full_state = None
+
     # ---- full-size moments (checkpoints) ----------------------------------------------------------------
     def _full_moments(self):
         """(m, v) over the whole flat buffer.  Sharded mode: needs `gather_state()` (a collective) beforehand."""
-        n = self.net.n_trainable_flat
         if self._shard is None:
             return self._m, self._v
         if self._full_state is None:
             raise RuntimeError("sharded FusedAdamW: call gather_state() on every rank before state_dict()")
-        return self._full_state
+        return self._full_state[:2]
 
     @torch.no_grad()
     def gather_state(self):
-        """Collective (every rank): assemble the full Adam moments from the shards, for `state_dict()`."""
+        """Collective (every rank): assemble the full Adam moments (and the EMA, unless the network holds it) from the
+        shards, for `state_dict()` / `ema_state_dict()`."""
         self._ensure_state()
         if self._shard is None:
             return
         rank, world, ranges = self._shard
         n = self.net.n_trainable_flat
-        full = [torch.zeros(n, dtype=torch.float32, device=self._m.device) for _ in range(2)]
-        owned = {(o + rank * (cnt // world)): (o, cnt) for o, cnt in ranges}
+        srcs = (self._m, self._v) + ((self._ema,) if self._ema is not None and not self._ema_swapped else ())
+        full = [torch.zeros(n, dtype=torch.float32, device=self._m.device) for _ in srcs]
         for (o, cnt, so) in self._segments:
-            for f, src in zip(full, (self._m, self._v)):
+            for f, src in zip(full, srcs):
                 f[o:o + cnt].copy_(src[so:so + cnt])
         for (o, cnt) in ranges:
             k = cnt // world
@@ -288,6 +405,7 @@ class ModelInterface(object):
         self.micro_batch = None       # samples per forward/backward pass (None: chosen from the free HBM, <= 64)
         self.max_grad_norm = 10.0     # reference model_interface.py:1121
         self.grad_bucket_elems = 64 * 1024 * 1024
+        self.ema_decay = None         # weight EMA kept by the fused optimizer (None: off); see ema_weights()
 
     def __repr__(self):
         return (f"{self.__class__.__name__} with {self.model.__class__.__name__} model with "
@@ -388,6 +506,12 @@ class ModelInterface(object):
             self.model.load_state_dict(checkpoint["model_state_dict"])
             if self.optimizer is not None:
                 self.optimizer.load_state_dict(checkpoint["optimizer_state_dict"])
+            if self._ema_on():
+                if "ema_state_dict" in checkpoint:
+                    self.optimizer.load_ema_state_dict(checkpoint["ema_state_dict"], checkpoint["ema_updates"])
+                else:
+                    self.optimizer.reset_ema()
+                    print("Info: the checkpoint has no weight EMA; the EMA starts from the loaded weights")
             if scheduler is not None:
                 scheduler.lambda_lr.load_state_dict(checkpoint["scheduler_state_dict"])
             epoch = checkpoint["epoch"]
@@ -400,17 +524,37 @@ class ModelInterface(object):
         return epoch, best_loss, scheduler
 
     def save_checkpoint(self, scheduler, epoch, best_loss, checkpoint_path):
+        if self._ema_on() and self.optimizer._ema_swapped:
+            # the network holds the EMA: model_state_dict would lose the live weights
+            raise RuntimeError("save_checkpoint() inside ema_weights()")
         sd = {k: v.detach().contiguous().cpu() for k, v in self.model.state_dict().items()}
-        torch.save(
-            {
-                "epoch": epoch,
-                "model_state_dict": sd,
-                "optimizer_state_dict": self.optimizer.state_dict(),
-                "scheduler_state_dict": (scheduler.lambda_lr.state_dict() if scheduler is not None else None),
-                "best_loss": best_loss,
-            },
-            checkpoint_path,
-        )
+        ck = {
+            "epoch": epoch,
+            "model_state_dict": sd,
+            "optimizer_state_dict": self.optimizer.state_dict(),
+            "scheduler_state_dict": (scheduler.lambda_lr.state_dict() if scheduler is not None else None),
+            "best_loss": best_loss,
+        }
+        if self._ema_on():   # the EMA in the model's state-dict format: UNet1d.load_state_dict takes it as it is
+            ck["ema_state_dict"] = self.optimizer.ema_state_dict(device="cpu")
+            ck["ema_updates"] = self.optimizer.ema_updates
+        torch.save(ck, checkpoint_path)
+
+    def _ema_on(self):
+        return isinstance(self.optimizer, FusedAdamW) and self.optimizer.ema_decay is not None
+
+    @contextlib.contextmanager
+    def ema_weights(self):
+        """Inside the context the network holds the EMA of its weights (`ema_decay`), so `sample`, `sample_windows`,
+        `predict_batch`, `predict_windows` and direct forward calls use it; the live weights are back, bit for bit, on
+        exit.  Under data parallelism every rank must enter it (the sharded EMA is all-gathered)."""
+        if not self._ema_on():
+            raise RuntimeError("no weight EMA: set ema_decay before the optimizer is created (training starts)")
+        self.optimizer.swap_ema()
+        try:
+            yield self.model
+        finally:
+            self.optimizer.swap_ema()
 
     def predict(self, dataloader, mixture_weights=(0.5, 0.5), num_steps=1000):
         self.model.eval()
@@ -446,11 +590,13 @@ class ModelInterface(object):
 
     def _set_optimizer(self, lr):
         if hasattr(self.model, "flat_params"):
-            self.optimizer = FusedAdamW(self.model, lr=lr)
+            self.optimizer = FusedAdamW(self.model, lr=lr, ema_decay=self.ema_decay)
             plan = self._shard_plan()
             if plan:
                 self.optimizer.set_sharding(torch.distributed.get_rank(), torch.distributed.get_world_size(), plan)
         else:  # an arbitrary user module (not the B200 denoiser): plain torch AdamW as in the reference
+            if self.ema_decay is not None:
+                raise ValueError("ema_decay needs a model with the flat-buffer API (the B200 UNet1d)")
             self.optimizer = torch.optim.AdamW(self.model.parameters(), lr=lr)
 
     def _set_lr(self, lr: float):

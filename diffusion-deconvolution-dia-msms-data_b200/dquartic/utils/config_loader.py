@@ -11,6 +11,7 @@ _OVERRIDES = {
     "batch_size": ("model", "batch_size"),
     "checkpoint_path": ("model", "checkpoint_path"),
     "use_wandb": ("wandb", "use_wandb"),
+    "ema_decay": ("model", "ema_decay"),   # optional key (absent: no weight EMA), not part of the default schema
 }
 
 

@@ -165,6 +165,11 @@ int dq_sumsq(const float* x, long n, double* out, void* stream);
 int dq_clip_coef(const double* sumsq, float max_norm, float gscale, float* out_norm_coef, void* stream);
 int dq_adamw(float* p, const float* g, float* m, float* v, long n, const float* coef_ptr, float lr, float b1, float b2,
              float eps, float wd, float step_size, float bc2_sqrt, void* stream);
+/* dq_adamw, then ema = ema + ema_w (p_new - ema) in the same pass (ema_w = 1 - EMA decay of this update) */
+int dq_adamw_ema(float* p, const float* g, float* m, float* v, float* ema, long n, const float* coef_ptr, float lr,
+                 float b1, float b2, float eps, float wd, float step_size, float bc2_sqrt, float ema_w, void* stream);
+/* exchange a[0:n) and b[0:n) in place */
+int dq_swap(float* a, float* b, long n, void* stream);
 int dq_fill(float* p, float v, long n, void* stream);
 
 /* ---- data path (utils/data_loader.py:70-88; model_interface.py:1071-1075) ----------------------------- */
