@@ -20,6 +20,7 @@ _SIGS = {
     "dq_add_mul": ("pffpls", 1),
     "dq_ddim_step": ("pppffffils", 1),
     "dq_ddim_step_x0": ("ppppffffils", 1),
+    "dq_dpm_step": ("pppppffiffffils", 1),
     "dq_scale_by": ("pppls", 1),
     "dq_cosine_sums": ("ppplis", 1),
     "dq_sample_finalize": ("ppppls", 1),

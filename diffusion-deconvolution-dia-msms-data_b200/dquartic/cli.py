@@ -1,7 +1,8 @@
 """`dquartic` command line — same commands and options as the reference (/root/reference/dquartic/cli.py:26-188):
 `dquartic train CONFIG [--parquet_directory --ms2-data-path --ms1-data-path --batch-size --checkpoint-path
 --use-wandb --threads]`, `dquartic generate-config`.  `--ema-decay` (model.ema_decay in the config) keeps an exponential
-moving average of the weights in the checkpoints.  Differences: `--batch-size/--threads` are cast to int (the
+moving average of the weights in the checkpoints.  `dquartic predict` (not in the reference) deconvolves a run of
+windows with a checkpoint.  Differences: `--batch-size/--threads` are cast to int (the
 reference passes strings to DataLoader and fails, SURVEY.md §5); under torchrun (RANK/WORLD_SIZE in the
 environment) each rank binds one GPU, joins an NCCL process group and trains a batch shard;
 `generate-train-data` (offline ETL) is out of scope.
@@ -10,9 +11,10 @@ import ast
 import os
 
 import click
+import numpy as np
 import torch
 
-from .model.model import DDIMDiffusionModel
+from .model.model import SAMPLERS, DDIMDiffusionModel
 from .model.unet1d import UNet1d
 from .utils.config_loader import generate_train_config, load_train_config
 from .utils.data_loader import DeviceBatchLoader, DIAMSDataset
@@ -45,6 +47,18 @@ def _init_distributed():
     torch.cuda.set_device(local)
     torch.distributed.init_process_group(backend="nccl" if torch.cuda.is_available() else "gloo")
     return rank, ws, local
+
+
+def _unet_from_config(config):
+    if config["model"]["use_model"] == "UNet1d":
+        u = config["model"]["UNet1d"]
+        return UNet1d(dim=u["dim"], channels=u["channels"], dim_mults=tuple(u["dim_mults"]),
+                      conditional=u["conditional"], init_cond_channels=u["init_cond_channels"],
+                      attn_cond_channels=u["attn_cond_channels"], tfer_dim_mult=u["tfer_dim_mult"],
+                      downsample_dim=u["downsample_dim"], simple=u["simple"])
+    if config["model"]["use_model"] == "CustomTransformer":
+        raise NotImplementedError("CustomTransformer is dead code under the reference's DDIM API (SURVEY.md finding 2)")
+    raise ValueError(f"Invalid model class: {config['model']['use_model']}")
 
 
 @cli.command()
@@ -96,16 +110,7 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
     data_loader = DeviceBatchLoader(dataset, per_rank, device, pool="hbm",
                                     batches_per_epoch=(len(dataset) + batch_size - 1) // batch_size)
 
-    if config["model"]["use_model"] == "UNet1d":
-        u = config["model"]["UNet1d"]
-        model = UNet1d(dim=u["dim"], channels=u["channels"], dim_mults=tuple(u["dim_mults"]),
-                       conditional=u["conditional"], init_cond_channels=u["init_cond_channels"],
-                       attn_cond_channels=u["attn_cond_channels"], tfer_dim_mult=u["tfer_dim_mult"],
-                       downsample_dim=u["downsample_dim"], simple=u["simple"]).to(device)
-    elif config["model"]["use_model"] == "CustomTransformer":
-        raise NotImplementedError("CustomTransformer is dead code under the reference's DDIM API (SURVEY.md finding 2)")
-    else:
-        raise ValueError(f"Invalid model class: {config['model']['use_model']}")
+    model = _unet_from_config(config).to(device)
     if world > 1:  # identical initial weights on every rank
         torch.distributed.broadcast(model.flat_params(), src=0)
         model.mark_params_modified()
@@ -137,6 +142,127 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
         wandb.finish()
     if world > 1:
         torch.distributed.destroy_process_group()
+
+
+PREDICT_SLICE_CHUNKS = 16   # windows handed to sample_windows at a time, in chunks: bounds the pinned host buffer
+
+
+def predict_to_file(diffusion_model, ms2, ms1, output, rank=0, world=1, sampler="dpm++2m", num_steps=20, seed=0,
+                    chunk=32):
+    """Deconvolve every window of `ms2` (N, rt, mz) conditioned on `ms1` (N, rt) into the .npy file `output`, float32
+    (N, rt, mz) in the input's intensity units.  Each window is min-max scaled on its own (MS2 and MS1 separately; a
+    zero range counts as 1), sampled with x_T from (seed, window index), and the prediction is scaled back with
+    pred * (max - min) + min.  This process samples the block `shard_windows(N, rank, world)`: rank 0 creates the
+    file, and under torch.distributed every rank writes its own slice after a barrier (no gather)."""
+    n = ms2.shape[0]
+    rt, mz = ms2.shape[1], ms2.shape[2]
+    dev = torch.device(diffusion_model.device)
+    dist = torch.distributed
+    on = dist.is_available() and dist.is_initialized()
+    if rank == 0:
+        np.lib.format.open_memmap(output, mode="w+", dtype=np.float32, shape=(n, rt, mz)).flush()
+    if on:
+        dist.barrier()
+    lo, hi = diffusion_model.shard_windows(n, rank, world)
+    if hi > lo:
+        dst = np.load(output, mmap_mode="r+")
+        ms2_min = np.empty(n, dtype=np.float32)
+        ms2_rng = np.empty(n, dtype=np.float32)
+
+        def scaled(raw):
+            # min and max on the host (no device sync: the previous chunk is still running), (x - min) / range in
+            # float64 on the device
+            flat = raw.reshape(raw.shape[0], -1)
+            mn = flat.min(1).astype(np.float64)
+            rng = flat.max(1).astype(np.float64) - mn
+            rng[rng == 0] = 1.0
+            shape = (-1,) + (1,) * (raw.ndim - 1)
+            x = torch.from_numpy(raw).to(dev).double()
+            x = (x - torch.from_numpy(mn).to(dev).view(shape)) / torch.from_numpy(rng).to(dev).view(shape)
+            return x.float(), mn, rng
+
+        def cond_fn(ids):   # ids: a contiguous run of window indices (sample_windows chunks the range it is given)
+            c2, mn, rng = scaled(np.ascontiguousarray(ms2[ids[0]:ids[-1] + 1]))
+            ms2_min[ids[0]:ids[-1] + 1] = mn
+            ms2_rng[ids[0]:ids[-1] + 1] = rng
+            return c2, scaled(np.ascontiguousarray(ms1[ids[0]:ids[-1] + 1]))[0]
+
+        step = PREDICT_SLICE_CHUNKS * chunk
+        buf = torch.empty((min(step, hi - lo), rt, mz), dtype=torch.float32).pin_memory()
+        for s in range(lo, hi, step):
+            e = min(s + step, hi)
+            _, maps = diffusion_model.sample_windows(list(range(s, e)), cond_fn, seed=seed, num_steps=num_steps,
+                                                     chunk=chunk, rank=0, world=1, out=buf[:e - s], sampler=sampler)
+            m = maps.numpy()
+            m *= ms2_rng[s:e, None, None]
+            m += ms2_min[s:e, None, None]
+            dst[s:e] = m
+        dst.flush()
+        del dst
+    if on:
+        dist.barrier()
+
+
+@cli.command()
+@click.argument("config-path", type=click.Path(exists=True, dir_okay=False), required=True)
+@click.option("--checkpoint-path", required=True, type=click.Path(exists=True, dir_okay=False),
+              help="Checkpoint written by `dquartic train`")
+@click.option("--ms2-data-path", required=True, type=click.Path(exists=True, dir_okay=False),
+              help="MS2 mixtures, .npy of shape (N, rt, mz), any numeric dtype")
+@click.option("--ms1-data-path", required=True, type=click.Path(exists=True, dir_okay=False),
+              help="MS1 conditioning, .npy of shape (N, rt)")
+@click.option("--output", required=True, type=click.Path(dir_okay=False),
+              help="Output .npy: the deconvolved maps, float32 (N, rt, mz), in input order and intensity units")
+@click.option("--sampler", default="dpm++2m", show_default=True, type=click.Choice(SAMPLERS))
+@click.option("--num-steps", default=20, show_default=True, type=int, help="Denoiser evaluations per window")
+@click.option("--seed", default=0, show_default=True, type=int, help="x_T of a window depends on (seed, its index)")
+@click.option("--chunk", default=32, show_default=True, type=click.IntRange(min=1), help="Windows per sampler batch")
+@click.option("--weights", default="auto", show_default=True, type=click.Choice(["auto", "ema", "model"]),
+              help="auto: the weight EMA when the checkpoint has one, else the trained weights")
+def predict(config_path, checkpoint_path, ms2_data_path, ms1_data_path, output, sampler, num_steps, seed, chunk,
+            weights):
+    """
+    Deconvolve the MS2 windows of a DIA run with a trained checkpoint.
+    """
+    config = load_train_config(config_path)
+    m = config["model"]
+    T = int(m["num_timesteps"])
+    ms2 = np.load(ms2_data_path, mmap_mode="r")
+    ms1 = np.load(ms1_data_path, mmap_mode="r")
+    if ms2.ndim != 3 or ms1.ndim != 2:
+        raise click.UsageError(f"expected MS2 (N, rt, mz) and MS1 (N, rt), got {ms2.shape} and {ms1.shape}")
+    if ms2.shape[0] != ms1.shape[0]:
+        raise click.UsageError(f"{ms2.shape[0]} MS2 windows but {ms1.shape[0]} MS1 chromatograms")
+    if ms2.shape[2] != m["UNet1d"]["downsample_dim"]:
+        raise click.UsageError(f"MS2 m/z axis is {ms2.shape[2]}, the model's downsample_dim is "
+                               f"{m['UNet1d']['downsample_dim']}")
+    if ms2.shape[1] != ms1.shape[1]:
+        raise click.UsageError(f"MS2 has {ms2.shape[1]} retention-time points, MS1 has {ms1.shape[1]}")
+    if not 2 <= num_steps <= T:
+        raise click.BadParameter(f"needs 2 <= num-steps <= {T}, got {num_steps}", param_hint="--num-steps")
+    ck = torch.load(checkpoint_path, map_location="cpu", mmap=True, weights_only=False)
+    if weights == "ema" and "ema_state_dict" not in ck:
+        raise click.UsageError(f"{checkpoint_path} has no ema_state_dict (train with --ema-decay to keep one)")
+    use_ema = weights == "ema" or (weights == "auto" and "ema_state_dict" in ck)
+
+    rank, world, local = _init_distributed()
+    if rank == 0:
+        click.echo(f"Info: sampling {ms2.shape[0]} windows with {sampler} x {num_steps} steps, "
+                   f"{'EMA' if use_ema else 'trained'} weights of {checkpoint_path}")
+    if not torch.cuda.is_available():
+        raise RuntimeError("the B200 build of dquartic has no CPU sampling path")
+    device = torch.device("cuda", local)
+    net = _unet_from_config(config)
+    net.load_state_dict(ck["ema_state_dict"] if use_ema else ck["model_state_dict"])
+    del ck
+    diffusion_model = DDIMDiffusionModel(
+        model_class=net.to(device), num_timesteps=T, beta_schedule_type=m["beta_schedule_type"],
+        pred_type=m["pred_type"], auto_normalize=m["auto_normalize"], device=device)
+    predict_to_file(diffusion_model, ms2, ms1, output, rank, world, sampler, num_steps, seed, chunk)
+    if world > 1:
+        torch.distributed.destroy_process_group()
+    if rank == 0:
+        click.echo(f"Info: wrote {output}")
 
 
 @cli.command()

@@ -62,6 +62,45 @@ def extract(a, t, x_shape):
     return out.reshape(b, *((1,) * (len(x_shape) - 1)))
 
 
+SAMPLERS = ("reference", "ddim", "dpm++2m")
+
+
+def sampler_grid(T, N):
+    """Time grid of the "ddim" / "dpm++2m" samplers: tau_i = rint((T-1) (1 - i/(N-1))^2), then raised so that the N
+    points strictly decrease from T-1 to 0 (every integer when N = T).  The quadratic spacing keeps the log-SNR jumps
+    at both ends of the cosine schedule small, where the reference's linear grid has its largest ones."""
+    T, N = int(T), int(N)
+    if not 2 <= N <= T:
+        raise ValueError(f"the ODE samplers take 2 <= num_steps <= {T}, got {N}")
+    tau = [int(np.rint((T - 1) * (1.0 - i / (N - 1)) ** 2)) for i in range(N)]
+    for i in range(N - 2, -1, -1):
+        tau[i] = max(tau[i], tau[i + 1] + 1)
+    return tau
+
+
+def ode_coefs(alpha_bars, taus, order):
+    """Per-step arguments (alpha, sigma, c_x, c_d, w_cur, w_prev, last) of `dq_dpm_step` over the grid `taus`, in float64
+    from the fp32 `alpha_bars` table.  Update i moves the state from tau_i to tau_{i+1} with h_i = lambda_{i+1} -
+    lambda_i, lambda = log(alpha / sigma): c_x = sigma_{i+1} / sigma_i, c_d = -alpha_{i+1} expm1(-h_i).  The first and
+    the final update (into tau = 0) are first order (w_cur = 1, w_prev = 0: DDIM with the true previous alpha_bar);
+    order 2 is DPM-Solver++(2M) (arXiv:2211.01095, Algorithm 2) in between, r = h_{i-1} / h_i, w_cur = 1 + 1/(2r),
+    w_prev = -1/(2r).  The last entry evaluates D at tau = 0 (`last` = 1)."""
+    ab = np.asarray(alpha_bars, dtype=np.float32).astype(np.float64)[list(taus)]
+    alpha, sigma = np.sqrt(ab), np.sqrt(1.0 - ab)
+    lam = np.log(alpha / sigma)
+    n = len(taus)
+    steps = []
+    for i in range(n - 1):
+        h = lam[i + 1] - lam[i]
+        w_cur, w_prev = 1.0, 0.0
+        if order == 2 and 0 < i < n - 2:
+            r = (lam[i] - lam[i - 1]) / h
+            w_cur, w_prev = 1.0 + 0.5 / r, -0.5 / r
+        steps.append((alpha[i], sigma[i], sigma[i + 1] / sigma[i], -alpha[i + 1] * math.expm1(-h), w_cur, w_prev, 0))
+    steps.append((alpha[-1], sigma[-1], 0.0, 0.0, 1.0, 0.0, 1))
+    return [tuple(float(v) for v in s[:6]) + (s[6],) for s in steps]
+
+
 def _sic_loss(x0_like, ms1_n):
     """MS1 summary-ion-chromatogram loss over the RT profiles (sum / mean / max over mz, each divided by its global
     maximum, MSE against the normalised MS1 chromatogram): see oracle/dquartic_oracle.py:sic_loss for the definition."""
@@ -191,13 +230,44 @@ class DDIMDiffusionModel(ModelInterface):
                x0_pred.numel())
         return x_prev, eps_pred
 
-    def sample(self, x_t, ms2_cond=None, ms1_cond=None, num_steps=1000):
+    def _ode_sample(self, x_t, ms2_cond, ms1_cond, num_steps, order):
+        """The "ddim" (order 1) / "dpm++2m" (order 2) loop: one model call and one fused `dq_dpm_step` per grid point,
+        every coefficient a host float fixed before the loop (so the loop captures into a CUDA graph).  Returns the
+        data prediction at tau = 0 and, when there is no MS2 conditioning to derive the noise map from, its epsilon."""
+        if self.pred_type not in ("eps", "x0"):
+            raise ValueError(f"Unknown pred_type: {self.pred_type}")
+        taus = sampler_grid(self.num_timesteps, num_steps)
+        steps = ode_coefs(self._ab_host, taus, order)
+        x = x_t.float().contiguous()
+        b, n = x.size(0), x.numel()
+        d_hist = torch.empty_like(x)
+        eps = torch.empty_like(x) if ms2_cond is None else None
+        for t, (alpha, sigma, c_x, c_d, w_cur, w_prev, last) in zip(taus, steps):
+            t_tensor = torch.full((b,), t, device=x.device, dtype=torch.long)
+            out = self.model(x, t_tensor, ms2_cond, ms1_cond).contiguous()
+            x_next = torch.empty_like(x)
+            N.call("dq_dpm_step", x, out, d_hist, x_next, eps if last else None, alpha, sigma,
+                   1 if self.pred_type == "x0" else 0, c_x, c_d, w_cur, w_prev, last, n)
+            x = x_next
+        return x, eps
+
+    def sample(self, x_t, ms2_cond=None, ms1_cond=None, num_steps=1000, sampler="reference"):
+        """Reverse process from x_t at t = T-1.  `sampler`: "reference" is the reference's loop bit for bit (its step
+        lands on alpha_bars[t-1] whatever the stride, so it only solves the ODE at num_steps = T); "ddim" and "dpm++2m"
+        solve the probability-flow ODE on `sampler_grid(T, num_steps)` with first / second order updates (`ode_coefs`)."""
+        if sampler not in SAMPLERS:
+            raise ValueError(f"unknown sampler {sampler!r}: expected one of {', '.join(SAMPLERS)}")
+        if sampler != "reference" and not 2 <= int(num_steps) <= self.num_timesteps:
+            raise ValueError(f"sampler {sampler!r} takes 2 <= num_steps <= {self.num_timesteps}, got {num_steps}")
         ms2_cond = self.normalize(ms2_cond) if ms2_cond is not None else None
         ms1_cond = self.normalize(ms1_cond) if ms1_cond is not None else None
         pred_noise = None
-        time_steps = torch.linspace(self.num_timesteps - 1, 0, num_steps, dtype=torch.long).tolist()
-        for t in time_steps:  # the step list lives on the host: no per-step device sync (reference: t.item())
-            x_t, pred_noise = self.p_sample(x_t, t, ms2_cond, ms1_cond)
+        if sampler != "reference":
+            x_t, pred_noise = self._ode_sample(x_t, ms2_cond, ms1_cond, int(num_steps), 2 if sampler == "dpm++2m" else 1)
+        else:
+            time_steps = torch.linspace(self.num_timesteps - 1, 0, num_steps, dtype=torch.long).tolist()
+            for t in time_steps:  # the step list lives on the host: no per-step device sync (reference: t.item())
+                x_t, pred_noise = self.p_sample(x_t, t, ms2_cond, ms1_cond)
         if ms2_cond is not None and self.auto_normalize and x_t.is_cuda:
             xo = torch.empty_like(x_t)
             pn = torch.empty_like(x_t)
@@ -223,7 +293,7 @@ class DDIMDiffusionModel(ModelInterface):
         return lo, lo + base + (1 if rank < rem else 0)
 
     def sample_windows(self, window_ids, cond_fn, seed=0, num_steps=50, chunk=32, rank=None, world=None, out=None,
-                       return_noise=False, cuda_graph=True):
+                       return_noise=False, cuda_graph=True, sampler="reference"):
         """DDIM-sample the DIA windows `window_ids` (model.py:293-324 per window; model_interface.py:1125-1150 returns
         item [0] only - here every window is kept).
 
@@ -234,7 +304,8 @@ class DDIMDiffusionModel(ModelInterface):
         seeded with `window_seed(seed, id)`.  Windows stream through the sampler `chunk` at a time; the 50-step loop of a
         full chunk is captured ONCE in a CUDA graph (fixed shapes: the scalar coefficients and timesteps of every step
         are baked in) and replayed per chunk; results are copied to pinned host memory on a side stream while the next
-        chunk runs.  Returns (ids of this rank, maps (n_local, rt, mz) on the host[, pred_noise])."""
+        chunk runs.  `sampler` is passed to `sample`.  Returns (ids of this rank, maps (n_local, rt, mz) on the
+        host[, pred_noise])."""
         dist = torch.distributed
         if rank is None or world is None:
             on = dist.is_available() and dist.is_initialized()
@@ -278,20 +349,21 @@ class DDIMDiffusionModel(ModelInterface):
                     c2.copy_(a)
                     c1.copy_(b1)
                     if cuda_graph and graph is None and n >= 2 * chunk:
-                        self.sample(xT.clone(), c2, c1, num_steps=min(2, num_steps))   # warm-up outside the capture
+                        self.sample(xT.clone(), c2, c1, num_steps=min(2, num_steps), sampler=sampler)   # warm-up outside the capture
                         torch.cuda.synchronize(dev)
                         graph = torch.cuda.CUDAGraph()
                         with torch.cuda.graph(graph):
-                            res = self.sample(xT, c2, c1, num_steps=num_steps)
+                            res = self.sample(xT, c2, c1, num_steps=num_steps, sampler=sampler)
                     if graph is not None:
                         graph.replay()
                         x, pn = res
                     else:
-                        x, pn = self.sample(xT, c2, c1, num_steps=num_steps)
+                        x, pn = self.sample(xT, c2, c1, num_steps=num_steps, sampler=sampler)
                 else:   # ragged last chunk: eager
                     xt = torch.empty((nb, rt, mz), dtype=torch.float32, device=dev)
                     draw_xT(cid, xt)
-                    x, pn = self.sample(xt, a.float().contiguous(), b1.float().contiguous(), num_steps=num_steps)
+                    x, pn = self.sample(xt, a.float().contiguous(), b1.float().contiguous(), num_steps=num_steps,
+                                        sampler=sampler)
                 cur = torch.cuda.current_stream(dev)
                 if graph is not None and nb == chunk:
                     # the graph's output buffers are overwritten by the next replay: move the results to staging buffers

@@ -422,7 +422,7 @@ class ModelInterface(object):
     def train_step(self, x_0, ms2_cond=None, ms1_cond=None, noise=None, ms1_loss_weight=0.0):
         raise NotImplementedError
 
-    def sample(self, x_t, ms2_cond=None, ms1_cond=None, num_steps=1000):
+    def sample(self, x_t, ms2_cond=None, ms1_cond=None, num_steps=1000, sampler="reference"):
         raise NotImplementedError
 
     def _ckpt_latest(self, checkpoint_path):
@@ -781,14 +781,16 @@ class ModelInterface(object):
                                              num_steps=num_steps)
         return sample[0].cpu().detach().numpy(), pred_noise[0].cpu().detach().numpy()
 
-    def predict_batch(self, x_T, ms2_cond, ms1_cond, num_steps=50, target=None):
+    def predict_batch(self, x_T, ms2_cond, ms1_cond, num_steps=50, target=None, sampler="reference"):
         """Batched multi-window prediction that keeps EVERY window (the reference's `_predict_one_batch` returns item
         [0] only, model_interface.py:1150).  With `target` (the clean maps, values in [0, 1]) it also returns the cheap
         evaluation metric of SURVEY.md §8f-2: the per-window cosine similarity between prediction and target, from one
-        fused pass (dq_cosine_sums).  Returns (pred, pred_noise) or (pred, pred_noise, cosine (b,))."""
+        fused pass (dq_cosine_sums).  `sampler` is passed to `sample`.  Returns (pred, pred_noise) or (pred, pred_noise,
+        cosine (b,))."""
         self.model.eval()
         with torch.no_grad():
-            pred, pred_noise = self.sample(x_T, ms2_cond=ms2_cond, ms1_cond=ms1_cond, num_steps=num_steps)
+            pred, pred_noise = self.sample(x_T, ms2_cond=ms2_cond, ms1_cond=ms1_cond, num_steps=num_steps,
+                                           sampler=sampler)
             if target is None:
                 return pred, pred_noise
             return pred, pred_noise, self.cosine_to_target(pred, target)
@@ -802,7 +804,7 @@ class ModelInterface(object):
                pred.numel() // b, b)
         return sums[:, 0] / (sums[:, 1].sqrt() * sums[:, 2].sqrt()).clamp_min(1e-30)
 
-    def predict_windows(self, dataloader, mixture_weights=(0.5, 0.5), num_steps=50, seed=0):
+    def predict_windows(self, dataloader, mixture_weights=(0.5, 0.5), num_steps=50, seed=0, sampler="reference"):
         """`predict` for throughput: every batch item is kept and scored.  Returns a list of dicts
         {ms2_1, ms1_1, mixture, pred, cosine} per batch (numpy arrays; `cosine` is pred vs ms2_1 per window)."""
         out = []
@@ -811,7 +813,8 @@ class ModelInterface(object):
         for ms2_1, ms1_1, ms2_2, ms1_2 in dataloader:
             x_0, ms1_cond, ms2_cond = self._mix_to_device(ms2_1, ms1_1, ms2_2, mixture_weights)
             x_T = torch.empty_like(x_0).normal_(generator=g)
-            pred, _, cos = self.predict_batch(x_T, ms2_cond, ms1_cond, num_steps=num_steps, target=x_0)
+            pred, _, cos = self.predict_batch(x_T, ms2_cond, ms1_cond, num_steps=num_steps, target=x_0,
+                                              sampler=sampler)
             out.append({"ms2_1": x_0.cpu().numpy(), "ms1_1": ms1_cond.cpu().numpy(), "mixture": ms2_cond.cpu().numpy(),
                         "pred": pred.cpu().numpy(), "cosine": cos.cpu().numpy()})
         return out

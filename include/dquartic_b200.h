@@ -34,6 +34,11 @@ int dq_ddim_step(const float* xt, const float* eps, float* xprev, float sa, floa
 /* pred_type "x0" reverse step (model.py:275-289): eps = (x_t - sa x0)/s1m, x_prev = last ? x0 : sap x0 + s1mp eps. */
 int dq_ddim_step_x0(const float* xt, const float* x0_pred, float* xprev, float* eps_out, float sa, float s1m, float sap,
                     float s1mp, int last, long n, void* stream);
+/* ODE sampler step (DDIM / DPM-Solver++(2M)): D = pred_x0 ? out : (x - sigma out)/alpha; last ? x_next = D (eps_out = eps)
+ * : x_next = c_x x + c_d (w_cur D + w_prev d_hist), d_hist = D. */
+int dq_dpm_step(const float* xt, const float* model_out, float* d_hist, float* x_next, float* eps_out, float alpha,
+                float sigma, int pred_x0, float c_x, float c_d, float w_cur, float w_prev, int last, long n,
+                void* stream);
 /* out[i] = x[i] * scale1[0] (scale read on the device: upstream gradient of the fused MSE node, 1 / world-size). */
 int dq_scale_by(const float* x, const float* scale1, float* out, long n, void* stream);
 /* evaluation metric (model_interface.py:630-667 consumer): out3[s] += {<a_s, b_s>, |a_s|^2, |b_s|^2} per window s. */

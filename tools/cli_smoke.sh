@@ -1,6 +1,7 @@
 #!/bin/bash
 # End-to-end smoke of the drop-in CLI on a GPU box: generate-config -> synthetic .npy pool -> `dquartic train` (2 epochs,
-# checkpoints in the reference format) -> resume from the latest checkpoint.  Shrunken m/z axis (640) so checkpoints stay small.
+# checkpoints in the reference format) -> resume from the latest checkpoint -> train with the weight EMA -> `dquartic predict`.
+# Shrunken m/z axis (640) so checkpoints stay small.
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)
 export PYTHONPATH=$ROOT/diffusion-deconvolution-dia-msms-data_b200:$PYTHONPATH
@@ -29,5 +30,17 @@ import torch
 ck = torch.load("ckpt/dquartic_latest_checkpoint.ckpt", map_location="cpu", weights_only=False)
 print("checkpoint keys", sorted(ck.keys()), "epoch", ck["epoch"], "n state entries", len(ck["model_state_dict"]))
 assert len(ck["model_state_dict"]) == 396
+PY
+# train with the weight EMA, then deconvolve the pool with it (--weights auto picks the EMA)
+mkdir -p ckpt_ema
+python -m dquartic.cli train --ms2-data-path ms2.npy --ms1-data-path ms1.npy --checkpoint-path ckpt_ema/best_model.ckpt \
+    --ema-decay 0.99 cfg.json 2>&1 | tail -3
+python -m dquartic.cli predict --checkpoint-path ckpt_ema/best_model.ckpt --ms2-data-path ms2.npy --ms1-data-path ms1.npy \
+    --output pred.npy --num-steps 10 --chunk 4 cfg.json
+python - <<'PY'
+import numpy as np
+p, ms2 = np.load("pred.npy"), np.load("ms2.npy")
+print("predicted", p.shape, p.dtype, "range", float(p.min()), float(p.max()))
+assert p.shape == ms2.shape and p.dtype == np.float32 and np.isfinite(p).all()
 PY
 echo CLI_SMOKE_OK
