@@ -178,6 +178,113 @@ __global__ void __launch_bounds__(256) cosine_sums_kernel(const float* __restric
   if (threadIdx.x < 3) atomicAdd(out + (size_t)s * 3 + threadIdx.x, tot);
 }
 
+// Validation scores of predicted maps p against clean maps g, (windows, rt, mz) fp32: per window the 9 float64 sums
+//   0 sse = sum (p - g)^2 ; 1-3 sum p g, sum p^2, sum g^2 ;
+//   4-6 sum_mz P G, sum P^2, sum G^2 with P[mz] = sum_rt p[rt, mz] (RT-summed spectra), G likewise ;
+//   7-8 sum_mz w r, sum_mz w over the m/z columns (XICs): r = Pearson correlation of p[:, mz] and g[:, mz] over RT,
+//       w = G[mz]; a column whose truth has no positive variance has w = 0, one whose prediction has none r = 0.
+// A thread owns 4 adjacent m/z columns and walks down RT (loads coalesced across the warp); column statistics are
+// float64 sums of x - x[rt = 0], so a constant column has exactly zero variance.  Padding columns past mz read as 0 and
+// add exact zeros.  The vector and the scalar kernel differ only in how they load: every sum is formed in the same
+// order, and a window's sums depend on nothing but its own data (no atomics, partials summed in block order by
+// map_scores_final_kernel), so they are bit-identical alone, in any batch and on every run.            8 B / element
+constexpr int kScoreThreads = 256;
+constexpr int kScoreCols = 4 * kScoreThreads;   // m/z columns per block
+constexpr int kScoreSlots = 9;
+
+template <bool VEC>
+__global__ void __launch_bounds__(kScoreThreads) map_scores_kernel(const float* __restrict__ pred,
+                                                                   const float* __restrict__ truth,
+                                                                   double* __restrict__ partial, int rt, int mz) {
+  __shared__ double red[(kScoreThreads / 32) * kScoreSlots];
+  const size_t base = (size_t)blockIdx.y * rt * mz;
+  const int c0 = blockIdx.x * kScoreCols + 4 * threadIdx.x;
+  const int nc = max(0, min(4, mz - c0));
+  double acc[kScoreSlots];
+#pragma unroll
+  for (int i = 0; i < kScoreSlots; ++i) acc[i] = 0.0;
+  if (nc > 0) {
+    auto load = [&](const float* src, int r, float (&v)[4]) {
+      const float* row = src + base + (size_t)r * mz + c0;
+      if (VEC) {
+        const float4 q = *reinterpret_cast<const float4*>(row);
+        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+      } else {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) v[j] = j < nc ? row[j] : 0.f;
+      }
+    };
+    float p0[4], g0[4];
+    load(pred, 0, p0);
+    load(truth, 0, g0);
+    double sp[4], sg[4], spp[4], sgg[4], spg[4], sse = 0.0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) sp[j] = sg[j] = spp[j] = sgg[j] = spg[j] = 0.0;
+#pragma unroll 4
+    for (int r = 0; r < rt; ++r) {
+      float p[4], g[4];
+      load(pred, r, p);
+      load(truth, r, g);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const double dp = (double)p[j] - (double)p0[j], dg = (double)g[j] - (double)g0[j];
+        const double d = (double)p[j] - (double)g[j];
+        sse = fma(d, d, sse);
+        sp[j] += dp;
+        sg[j] += dg;
+        spp[j] = fma(dp, dp, spp[j]);
+        sgg[j] = fma(dg, dg, sgg[j]);
+        spg[j] = fma(dp, dg, spg[j]);
+      }
+    }
+    acc[0] = sse;
+    const double n = (double)rt;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const double a = p0[j], b = g0[j];
+      const double P = fma(n, a, sp[j]), G = fma(n, b, sg[j]);
+      // sum (dp + a)(dg + b), sum (dp + a)^2, sum (dg + b)^2; explicit fma so that no contraction choice of the
+      // compiler can differ between the two kernels
+      acc[1] += fma(n * a, b, fma(b, sp[j], fma(a, sg[j], spg[j])));
+      acc[2] += fma(n * a, a, fma(2.0 * a, sp[j], spp[j]));
+      acc[3] += fma(n * b, b, fma(2.0 * b, sg[j], sgg[j]));
+      acc[4] = fma(P, G, acc[4]);
+      acc[5] = fma(P, P, acc[5]);
+      acc[6] = fma(G, G, acc[6]);
+      const double varg = sgg[j] - sg[j] * sg[j] / n;
+      if (varg > 0.0) {
+        const double varp = spp[j] - sp[j] * sp[j] / n;
+        double r = 0.0;
+        if (varp > 0.0) r = fmin(1.0, fmax(-1.0, (spg[j] - sp[j] * sg[j] / n) / (sqrt(varp) * sqrt(varg))));
+        acc[7] = fma(G, r, acc[7]);
+        acc[8] += G;
+      }
+    }
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int i = 0; i < kScoreSlots; ++i) {
+    const double s = warp_sum_d(acc[i]);
+    if (lane == 0) red[warp * kScoreSlots + i] = s;
+  }
+  __syncthreads();
+  if (threadIdx.x < kScoreSlots) {
+    double s = 0.0;
+    for (int w = 0; w < kScoreThreads / 32; ++w) s += red[w * kScoreSlots + threadIdx.x];
+    partial[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * kScoreSlots + threadIdx.x] = s;
+  }
+}
+
+// out9[w] = sum over the column blocks of window w, in block order
+__global__ void __launch_bounds__(32) map_scores_final_kernel(const double* __restrict__ partial,
+                                                             double* __restrict__ out9, int nblk) {
+  if (threadIdx.x >= kScoreSlots) return;
+  const double* src = partial + (size_t)blockIdx.x * nblk * kScoreSlots + threadIdx.x;
+  double s = 0.0;
+  for (int b = 0; b < nblk; ++b) s += src[(size_t)b * kScoreSlots];
+  out9[(size_t)blockIdx.x * kScoreSlots + threadIdx.x] = s;
+}
+
 // tail of sample(): x = (x+1)*0.5 ; pred_noise = (cond_n+1)*0.5 - x      (model.py:319-322)
 __global__ void __launch_bounds__(256) sample_finalize_kernel(const float* __restrict__ x, const float* __restrict__ cond_n,
                                                               float* __restrict__ xo, float* __restrict__ pn, long n) {
@@ -284,6 +391,30 @@ DQ_API int dq_cosine_sums(const float* a, const float* b, float* out3, long n_pe
   if (bx > 256) bx = 256;
   dim3 grid((unsigned)bx, (unsigned)n_samples);
   cosine_sums_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(a, b, out3, n_per_sample);
+  DQ_LAUNCH_CHECK();
+  return 0;
+}
+DQ_API int dq_map_scores_nblk(int mz) { return mz > 0 ? (mz + kScoreCols - 1) / kScoreCols : 0; }
+DQ_API int dq_map_scores(const float* pred, const float* truth, double* partial, double* out9, int n_windows, int rt,
+                         int mz, void* stream) {
+  if (n_windows <= 0) return 0;
+  if (rt <= 0 || mz <= 0) return -2;
+  const int nblk = dq_map_scores_nblk(mz);
+  const bool vec = (mz & 3) == 0 && ((((size_t)pred) | ((size_t)truth)) & 15) == 0;
+  const size_t per = (size_t)rt * mz;
+  for (int w0 = 0; w0 < n_windows; w0 += 65535) {   // gridDim.y limit
+    const int nw = n_windows - w0 < 65535 ? n_windows - w0 : 65535;
+    const dim3 grid((unsigned)nblk, (unsigned)nw);
+    double* part = partial + (size_t)w0 * nblk * kScoreSlots;
+    if (vec)
+      map_scores_kernel<true><<<grid, kScoreThreads, 0, (cudaStream_t)stream>>>(pred + w0 * per, truth + w0 * per, part,
+                                                                               rt, mz);
+    else
+      map_scores_kernel<false><<<grid, kScoreThreads, 0, (cudaStream_t)stream>>>(pred + w0 * per, truth + w0 * per,
+                                                                                part, rt, mz);
+    DQ_LAUNCH_CHECK();
+  }
+  map_scores_final_kernel<<<(unsigned)n_windows, 32, 0, (cudaStream_t)stream>>>(partial, out9, nblk);
   DQ_LAUNCH_CHECK();
   return 0;
 }

@@ -23,6 +23,7 @@ _SIGS = {
     "dq_dpm_step": ("pppppffiffffils", 1),
     "dq_scale_by": ("pppls", 1),
     "dq_cosine_sums": ("ppplis", 1),
+    "dq_map_scores": ("ppppiiis", 2),
     "dq_sample_finalize": ("ppppls", 1),
     "dq_mse": ("ppppfls", 1),
     "dq_add_inplace": ("ppls", 1),
@@ -93,6 +94,8 @@ def lib():
             fn.argtypes = [_CT[c] for c in sig]
         _lib.dq_la_nchunk.restype = ctypes.c_int
         _lib.dq_la_nchunk.argtypes = [ctypes.c_int]
+        _lib.dq_map_scores_nblk.restype = ctypes.c_int
+        _lib.dq_map_scores_nblk.argtypes = [ctypes.c_int]
         _lib.dq_gemm_last_error.restype = ctypes.c_int
         _lib.dq_gemm_last_error.argtypes = []
         _lib.dq_la_tc_last_error.restype = ctypes.c_int
@@ -101,7 +104,7 @@ def lib():
 
 
 def exported_symbols():
-    return sorted(list(_SIGS) + ["dq_la_nchunk", "dq_gemm_last_error", "dq_la_tc_last_error"])
+    return sorted(list(_SIGS) + ["dq_la_nchunk", "dq_map_scores_nblk", "dq_gemm_last_error", "dq_la_tc_last_error"])
 
 
 def _ptr(x):
@@ -117,7 +120,7 @@ def _ptr(x):
 
 
 _OK_DTYPES = (torch.float32, torch.bfloat16, torch.int32, torch.int64)
-_F64_ARGS = {"dq_sumsq", "dq_clip_coef", "dq_mse"}   # the only entry points with a double* (accumulators)
+_F64_ARGS = {"dq_sumsq", "dq_clip_coef", "dq_mse", "dq_map_scores"}   # the only entry points with a double* (accumulators)
 
 
 def call(name, *args, allow=()):
@@ -178,6 +181,11 @@ def _cuda_err(rc):
 
 def la_nchunk(L):
     return int(lib().dq_la_nchunk(int(L)))
+
+
+def map_scores_nblk(mz):
+    """Column blocks of dq_map_scores per window: its scratch holds n_windows * map_scores_nblk(mz) * 9 doubles."""
+    return int(lib().dq_map_scores_nblk(int(mz)))
 
 
 def la_tc_last_error():

@@ -1,8 +1,10 @@
 """`dquartic` command line — same commands and options as the reference (/root/reference/dquartic/cli.py:26-188):
 `dquartic train CONFIG [--parquet_directory --ms2-data-path --ms1-data-path --batch-size --checkpoint-path
 --use-wandb --threads]`, `dquartic generate-config`.  `--ema-decay` (model.ema_decay in the config) keeps an exponential
-moving average of the weights in the checkpoints.  `dquartic predict` (not in the reference) deconvolves a run of
-windows with a checkpoint.  Differences: `--batch-size/--threads` are cast to int (the
+moving average of the weights in the checkpoints.  `--validation-fraction` (the optional config section "validation")
+holds out slices and selects the best checkpoint by a held-out denoising loss.  `dquartic predict` (not in the
+reference) deconvolves a run of windows with a checkpoint; `dquartic evaluate` scores a checkpoint on the held-out
+mixtures.  Differences: `--batch-size/--threads` are cast to int (the
 reference passes strings to DataLoader and fails, SURVEY.md §5); under torchrun (RANK/WORLD_SIZE in the
 environment) each rank binds one GPU, joins an NCCL process group and trains a batch shard;
 `generate-train-data` (offline ETL) is out of scope.
@@ -18,6 +20,7 @@ from .model.model import SAMPLERS, DDIMDiffusionModel
 from .model.unet1d import UNet1d
 from .utils.config_loader import generate_train_config, load_train_config
 from .utils.data_loader import DeviceBatchLoader, DIAMSDataset
+from .utils.validation import ValidationSet, check_section, hold_out, validation_pairs
 
 
 class PythonLiteralOption(click.Option):
@@ -73,8 +76,11 @@ def _unet_from_config(config):
 @click.option("--ema-decay", default=None, type=click.FloatRange(0.0, 1.0, min_open=True, max_open=True),
               help="Keep an exponential moving average of the weights with this decay (e.g. 0.9999) and save it in the "
                    "checkpoints as ema_state_dict, overrides config file")
+@click.option("--validation-fraction", default=None, type=float,
+              help="Hold out this fraction of the slices (0 < f < 1, the last ones in file order) and select the best "
+                   "checkpoint by their denoising loss, overrides validation.fraction of the config file")
 def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_size, checkpoint_path, use_wandb, threads,
-          ema_decay):
+          ema_decay, validation_fraction):
     """
     Train a DDIM model on the DIAMS dataset.
     """
@@ -93,7 +99,9 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
 
     config = load_train_config(config_path, parquet_directory=parquet_directory, ms2_data_path=ms2_data_path,
                                ms1_data_path=ms1_data_path, batch_size=batch_size, checkpoint_path=checkpoint_path,
-                               use_wandb=use_wandb, threads=threads, ema_decay=ema_decay)
+                               use_wandb=use_wandb, threads=threads, ema_decay=ema_decay,
+                               validation_fraction=validation_fraction)
+    val_cfg = _validation_section(config, for_train=True)
     batch_size = int(config["model"]["batch_size"])
     checkpoint_path = config["model"]["checkpoint_path"]
     use_wandb = config["wandb"]["use_wandb"]
@@ -103,12 +111,14 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
     device = torch.device("cuda", local)
     dataset = DIAMSDataset(config["data"]["parquet_directory"], config["data"]["ms2_data_path"],
                            config["data"]["ms1_data_path"], normalize=config["data"]["normalize"])
+    if val_cfg is not None:
+        val_pairs = _validation_pairs(dataset, val_cfg)
     if world > 1:
         import random
         random.seed(1234 + rank)  # each rank draws its own pairs, like DataLoader workers do in the reference
     per_rank = max(1, batch_size // world)
     data_loader = DeviceBatchLoader(dataset, per_rank, device, pool="hbm",
-                                    batches_per_epoch=(len(dataset) + batch_size - 1) // batch_size)
+                                    batches_per_epoch=(dataset.n_train + batch_size - 1) // batch_size)
 
     model = _unet_from_config(config).to(device)
     if world > 1:  # identical initial weights on every rank
@@ -126,6 +136,9 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
         device=device)
     diffusion_model.micro_batch = int(os.environ.get("DQUARTIC_MICRO_BATCH", "0")) or None
     diffusion_model.ema_decay = config["model"].get("ema_decay")
+    if val_cfg is not None:
+        diffusion_model.validation = ValidationSet(data_loader, val_pairs, config["model"]["num_timesteps"],
+                                                   val_cfg["bands"], val_cfg["seed"], val_cfg["every_n_epochs"])
 
     if use_wandb and rank == 0:
         import wandb
@@ -142,6 +155,25 @@ def train(config_path, parquet_directory, ms2_data_path, ms1_data_path, batch_si
         wandb.finish()
     if world > 1:
         torch.distributed.destroy_process_group()
+
+
+def _validation_section(config, for_train):
+    """The config's "validation" section range-checked with its defaults filled in, or None when it is absent."""
+    if "validation" not in config:
+        return None
+    try:
+        return check_section(config["validation"], for_train)
+    except ValueError as e:
+        raise click.BadParameter(str(e), param_hint="--validation-fraction / the config's validation section")
+
+
+def _validation_pairs(dataset, val_cfg):
+    """Hold out the config's fraction of `dataset` and draw the fixed validation pairs (host only)."""
+    try:
+        lo, hi = hold_out(dataset, val_cfg["fraction"])
+        return validation_pairs(dataset, lo, hi, val_cfg["windows"], val_cfg["seed"])
+    except ValueError as e:
+        raise click.UsageError(str(e))
 
 
 PREDICT_SLICE_CHUNKS = 16   # windows handed to sample_windows at a time, in chunks: bounds the pinned host buffer
@@ -263,6 +295,95 @@ def predict(config_path, checkpoint_path, ms2_data_path, ms1_data_path, output, 
         torch.distributed.destroy_process_group()
     if rank == 0:
         click.echo(f"Info: wrote {output}")
+
+
+def evaluate_model(diffusion_model, vset, sampler="dpm++2m", num_steps=20, seed=0, chunk=32, rank=None, world=None):
+    """Score the current weights of `diffusion_model` on the validation set `vset`: the held-out denoising loss per band
+    (`validate`) and, unless `num_steps` is 0, the maps `sampler` draws in `num_steps` steps against the clean maps
+    (`score_samples`).  Every rank of a process group must call it; each returns the full result.  Returns a
+    JSON-ready dict {"loss_by_band", "val_loss"[, "samplers": {"<sampler>@<steps>": {"mean", "per_window"}}]}."""
+    v = diffusion_model.validate(vset, chunk=chunk, rank=rank, world=world)
+    out = {"loss_by_band": [float(x) for x in v["loss_by_band"]], "val_loss": v["val_loss"]}
+    if num_steps:
+        s = diffusion_model.score_samples(vset, sampler=sampler, num_steps=num_steps, seed=seed, chunk=chunk,
+                                          rank=rank, world=world)
+        out["samplers"] = {f"{sampler}@{num_steps}": {
+            "mean": s["mean"], "per_window": {k: [float(x) for x in a] for k, a in s["per_window"].items()}}}
+    return out
+
+
+@cli.command()
+@click.argument("config-path", type=click.Path(exists=True, dir_okay=False), required=True)
+@click.option("--checkpoint-path", required=True, type=click.Path(exists=True, dir_okay=False),
+              help="Checkpoint written by `dquartic train`")
+@click.option("--parquet_directory", default=None, help="Directory of Parquet slices, overrides config file")
+@click.option("--ms2-data-path", default=None, help="Path to MS2 data, overrides config file")
+@click.option("--ms1-data-path", default=None, help="Path to MS1 data, overrides config file")
+@click.option("--validation-fraction", default=None, type=float,
+              help="Held-out fraction of the slices (0 < f <= 1; 1 scores whole files), overrides validation.fraction "
+                   "of the config file")
+@click.option("--weights", default="auto", show_default=True, type=click.Choice(["auto", "ema", "model", "both"]),
+              help="auto: the weight EMA when the checkpoint has one, else the trained weights; both: each in turn")
+@click.option("--sampler", default="dpm++2m", show_default=True, type=click.Choice(SAMPLERS))
+@click.option("--num-steps", default=20, show_default=True, type=int,
+              help="Denoiser evaluations per sampled map; 0: the denoising loss only")
+@click.option("--seed", default=0, show_default=True, type=int, help="x_T of a window depends on (seed, its index)")
+@click.option("--chunk", default=32, show_default=True, type=click.IntRange(min=1), help="Windows per batch")
+@click.option("--output", default=None, type=click.Path(dir_okay=False), help="JSON file (default: stdout)")
+def evaluate(config_path, checkpoint_path, parquet_directory, ms2_data_path, ms1_data_path, validation_fraction, weights,
+             sampler, num_steps, seed, chunk, output):
+    """
+    Score a checkpoint on the held-out validation mixtures: denoising loss per timestep band and sampled-map scores.
+    """
+    import json
+
+    config = load_train_config(config_path, parquet_directory=parquet_directory, ms2_data_path=ms2_data_path,
+                               ms1_data_path=ms1_data_path, validation_fraction=validation_fraction)
+    val_cfg = _validation_section(config, for_train=False)
+    if val_cfg is None:
+        raise click.UsageError("the config has no validation section: pass --validation-fraction")
+    m = config["model"]
+    T = int(m["num_timesteps"])
+    if num_steps != 0 and not 2 <= num_steps <= T:
+        raise click.BadParameter(f"needs 0 or 2 <= num-steps <= {T}, got {num_steps}", param_hint="--num-steps")
+    ck = torch.load(checkpoint_path, map_location="cpu", mmap=True, weights_only=False)
+    has_ema = "ema_state_dict" in ck
+    if weights in ("ema", "both") and not has_ema:
+        raise click.UsageError(f"{checkpoint_path} has no ema_state_dict (train with --ema-decay to keep one)")
+    names = {"auto": ["ema" if has_ema else "model"], "ema": ["ema"], "model": ["model"], "both": ["model", "ema"]}[weights]
+    dataset = DIAMSDataset(config["data"]["parquet_directory"], config["data"]["ms2_data_path"],
+                           config["data"]["ms1_data_path"], normalize=config["data"]["normalize"])
+    if dataset.ms2_data.shape[2] != m["UNet1d"]["downsample_dim"]:
+        raise click.UsageError(f"MS2 m/z axis is {dataset.ms2_data.shape[2]}, the model's downsample_dim is "
+                               f"{m['UNet1d']['downsample_dim']}")
+    pairs = _validation_pairs(dataset, val_cfg)
+
+    rank, world, local = _init_distributed()
+    if not torch.cuda.is_available():
+        raise RuntimeError("the B200 build of dquartic has no CPU evaluation path")
+    device = torch.device("cuda", local)
+    loader = DeviceBatchLoader(dataset, 1, device, pool="hbm")
+    vset = ValidationSet(loader, pairs, T, val_cfg["bands"], val_cfg["seed"], val_cfg["every_n_epochs"])
+    net = _unet_from_config(config).to(device)
+    diffusion_model = DDIMDiffusionModel(
+        model_class=net, num_timesteps=T, beta_schedule_type=m["beta_schedule_type"], pred_type=m["pred_type"],
+        auto_normalize=m["auto_normalize"], device=device)
+    result = {"checkpoint": checkpoint_path, "weights": names, "windows": vset.windows, "bands": vset.bands,
+              "results": {}}
+    for name in names:
+        net.load_state_dict(ck["ema_state_dict"] if name == "ema" else ck["model_state_dict"])
+        result["results"][name] = evaluate_model(diffusion_model, vset, sampler, num_steps, seed, chunk)
+        if rank == 0:
+            click.echo(f"Info: {name} weights: val_loss={result['results'][name]['val_loss']}", err=True)
+    if rank == 0:
+        text = json.dumps(result)
+        if output is None:
+            click.echo(text)
+        else:
+            with open(output, "w") as f:
+                f.write(text + "\n")
+    if world > 1:
+        torch.distributed.destroy_process_group()
 
 
 @cli.command()

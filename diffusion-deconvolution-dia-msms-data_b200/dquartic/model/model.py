@@ -390,6 +390,25 @@ class DDIMDiffusionModel(ModelInterface):
             e.synchronize()
         return (ids, out, out_noise) if return_noise else (ids, out)
 
+    # ------------------------------------------------------------------------------------------ validation
+    @torch.no_grad()
+    def denoising_loss(self, x0, ms2_cond, ms1_cond, t, noise):
+        """Per-sample MSE of the network's own training target at given timesteps `t` (b,) and standard-normal `noise`
+        (b, rt, mz), no gradient: x_t = dq_qsample(x0, t, noise) (with the auto-normalise of `train_step`), one forward
+        pass, target = noise ("eps") or normalize(x0) ("x0"), squared error summed by dq_map_scores.  Without the
+        `loss_weight[t]` factor and without the MS1 SIC term of `train_step`.  Returns (b,) float64."""
+        if self.pred_type not in ("eps", "x0"):
+            raise ValueError(f"Unknown pred_type: {self.pred_type}")
+        x0 = x0.float().contiguous()
+        noise = noise.float().contiguous()
+        t = t.to(x0.device).long().contiguous()
+        ms2_n = self.normalize(ms2_cond) if ms2_cond is not None else None
+        ms1_n = self.normalize(ms1_cond) if ms1_cond is not None else None
+        x_t = self._q_sample_fused(x0, t, noise)
+        pred = self.model(x_t, t, ms2_n, ms1_n)
+        target = noise if self.pred_type == "eps" else self.normalize(x0)
+        return self.map_scores(pred, target)[:, 0] / (x0[0].numel())
+
     # ------------------------------------------------------------------------------------------ training step
     def train_step(self, x_0, ms2_cond=None, ms1_cond=None, noise=None, ms1_loss_weight=0.0, t=None):
         """model.py:326-406.  `t` (optional, not in the reference) injects the timesteps for parity tests."""

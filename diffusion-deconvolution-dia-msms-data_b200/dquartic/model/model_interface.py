@@ -406,6 +406,8 @@ class ModelInterface(object):
         self.max_grad_norm = 10.0     # reference model_interface.py:1121
         self.grad_bucket_elems = 64 * 1024 * 1024
         self.ema_decay = None         # weight EMA kept by the fused optimizer (None: off); see ema_weights()
+        self.validation = None        # a dquartic.utils.validation.ValidationSet (None: off); see validate()
+        self.val_history = []         # one dict per validated epoch
 
     def __repr__(self):
         return (f"{self.__class__.__name__} with {self.model.__class__.__name__} model with "
@@ -436,6 +438,7 @@ class ModelInterface(object):
         start_epoch, best_loss, lr_scheduler = self.load_checkpoint(lr_scheduler, self._ckpt_latest(checkpoint_path),
                                                                     self.device)
         best_epoch = start_epoch
+        vset = self.validation
         if start_epoch > 0:
             # resumed run: do not replay the (t, noise) stream of the first epochs; every rank keeps its own stream
             rank = torch.distributed.get_rank() if self._dist_on() else 0
@@ -453,17 +456,23 @@ class ModelInterface(object):
             if use_wandb and self._is_rank0():
                 import wandb
                 wandb.log({"epoch": epoch, "train/loss": avg, "learning_rate": lr_now})
+            # with validation the held-out loss (the EMA's when the EMA is on) selects the best checkpoint, and only
+            # epochs that ran it can become the best; without it, the epoch-mean training loss does
+            metric, val_kw = avg, {}
+            if vset is not None:
+                metric = self._validate_epoch(epoch, use_wandb) if vset.due(epoch) else None
+                val_kw = {"val_loss": metric}
             if isinstance(self.optimizer, FusedAdamW):
                 self.optimizer.gather_state()   # sharded optimizer: collective, every rank (no-op otherwise)
+            better = metric is not None and metric < best_loss
+            if better:
+                best_loss, best_epoch = metric, epoch + 1
             if self._is_rank0():
                 print(f"[Training] Epoch={epoch+1}, lr={lr_now}, loss={avg}")
-                self.save_checkpoint(lr_scheduler, epoch, avg, self._ckpt_latest(checkpoint_path))
-                if avg < best_loss:
-                    best_loss = avg
-                    best_epoch = epoch + 1
-                    self.save_checkpoint(lr_scheduler, epoch, best_loss, checkpoint_path)
-            elif avg < best_loss:
-                best_loss, best_epoch = avg, epoch + 1
+                self.save_checkpoint(lr_scheduler, epoch, avg if vset is None else best_loss,
+                                     self._ckpt_latest(checkpoint_path), **val_kw)
+                if better:
+                    self.save_checkpoint(lr_scheduler, epoch, best_loss, checkpoint_path, **val_kw)
             if use_wandb and (epoch == 0 or epoch % log_every_n_epochs == 0) and self._is_rank0():
                 # the reference logs a plotted prediction here (model_interface.py:440-448); plotting is out of scope of
                 # this build, so the training loop must not die on it (a raise here would kill rank 0 after the first
@@ -480,6 +489,31 @@ class ModelInterface(object):
                 break
         if self._is_rank0():
             print(f"Best model checkpoint saved at epoch {best_epoch} with loss: {best_loss:.6f}")
+
+    def _validate_epoch(self, epoch, use_wandb):
+        """`validate` on the live weights and, with the EMA on, inside `ema_weights()` (every rank); records, prints and
+        logs them.  Returns the selection metric: the EMA's val_loss when the EMA is on, else the live one."""
+        vset = self.validation
+        live = self.validate(vset)
+        rec = {"epoch": epoch + 1, "val_loss": live["val_loss"], "loss_by_band": live["loss_by_band"]}
+        metric = live["val_loss"]
+        if self._ema_on():
+            with self.ema_weights():
+                ema = self.validate(vset)
+            rec.update(ema_val_loss=ema["val_loss"], ema_loss_by_band=ema["loss_by_band"])
+            metric = ema["val_loss"]
+        self.val_history.append(rec)
+        if self._is_rank0():
+            ema_txt = f", ema_val_loss={rec['ema_val_loss']}" if "ema_val_loss" in rec else ""
+            print(f"[Validation] Epoch={epoch + 1}, val_loss={rec['val_loss']}{ema_txt}")
+            if use_wandb:
+                import wandb
+                log = {"epoch": epoch, "val/loss": rec["val_loss"]}
+                log.update({f"val/loss_t{t}": float(v) for t, v in zip(vset.bands, rec["loss_by_band"])})
+                if "ema_val_loss" in rec:
+                    log["val_ema/loss"] = rec["ema_val_loss"]
+                wandb.log(log)
+        return metric
 
     def train_with_warmup(self, dataloader, num_epochs, num_warmup_steps=5, learning_rate=1e-4, use_wandb=True,
                           log_every_n_epochs=100, checkpoint_path="best_model.ckpt"):
@@ -516,6 +550,12 @@ class ModelInterface(object):
                 scheduler.lambda_lr.load_state_dict(checkpoint["scheduler_state_dict"])
             epoch = checkpoint["epoch"]
             best_loss = checkpoint["best_loss"]
+            if ("val_loss" in checkpoint) != (self.validation is not None):
+                # a training loss and a held-out loss are not comparable: the best checkpoint is chosen afresh
+                print(f"Info: the checkpoint's best loss is a {'validation' if 'val_loss' in checkpoint else 'training'} "
+                      f"loss but this run selects by {'validation' if self.validation is not None else 'training'} "
+                      "loss; the best loss restarts at inf")
+                best_loss = float("inf")
             print(f"Resumed from ({checkpoint_path}) epoch {epoch}, best loss {best_loss:.6f}")
         else:
             print(f"No checkpoint ({checkpoint_path}) found. Starting from scratch.")
@@ -523,7 +563,8 @@ class ModelInterface(object):
             best_loss = float("inf")
         return epoch, best_loss, scheduler
 
-    def save_checkpoint(self, scheduler, epoch, best_loss, checkpoint_path):
+    def save_checkpoint(self, scheduler, epoch, best_loss, checkpoint_path, **extra):
+        """Writes the reference's checkpoint dictionary; `extra` keys (validation: `val_loss`) are added to it."""
         if self._ema_on() and self.optimizer._ema_swapped:
             # the network holds the EMA: model_state_dict would lose the live weights
             raise RuntimeError("save_checkpoint() inside ema_weights()")
@@ -538,6 +579,7 @@ class ModelInterface(object):
         if self._ema_on():   # the EMA in the model's state-dict format: UNet1d.load_state_dict takes it as it is
             ck["ema_state_dict"] = self.optimizer.ema_state_dict(device="cpu")
             ck["ema_updates"] = self.optimizer.ema_updates
+        ck.update(extra)
         torch.save(ck, checkpoint_path)
 
     def _ema_on(self):
@@ -803,6 +845,104 @@ class ModelInterface(object):
         N.call("dq_cosine_sums", pred.float().contiguous(), target.to(pred.device).float().contiguous(), sums,
                pred.numel() // b, b)
         return sums[:, 0] / (sums[:, 1].sqrt() * sums[:, 2].sqrt()).clamp_min(1e-30)
+
+    @staticmethod
+    def map_scores(pred, truth):
+        """The 9 float64 sums of `dq_map_scores` per window of (b, rt, mz) maps, one deterministic pass: sse, <p, g>,
+        |p|^2, |g|^2, the same three of the RT-summed spectra, and the weighted XIC correlation sums.  Turn them into
+        scores with `dquartic.utils.validation.finalize_scores`.  Returns (b, 9) float64 on the maps' device."""
+        if pred.dim() != 3 or tuple(pred.shape) != tuple(truth.shape):
+            raise ValueError(f"map_scores needs two (b, rt, mz) maps of one shape, got {tuple(pred.shape)} and "
+                             f"{tuple(truth.shape)}")
+        b, rt, mz = pred.shape
+        pred = pred.float().contiguous()
+        truth = truth.to(pred.device).float().contiguous()
+        part = torch.empty(b * N.map_scores_nblk(mz) * 9, dtype=torch.float64, device=pred.device)
+        out = torch.empty(b, 9, dtype=torch.float64, device=pred.device)
+        N.call("dq_map_scores", pred, truth, part, out, b, rt, mz)
+        return out
+
+    def _gather_windows(self, local, n_windows, rank, world):
+        """Per-window rows (n_local, k) of this rank's `shard_windows` block -> all (n_windows, k) rows in window order on
+        every rank (padded all-gather) when a process group is up; otherwise the local block as it is."""
+        dist = torch.distributed
+        if not (dist.is_available() and dist.is_initialized()) or world == 1:
+            return local
+        width = -(-n_windows // world)
+        buf = torch.zeros(width, local.shape[1], dtype=local.dtype, device=self.device)
+        buf[:local.shape[0]].copy_(local)
+        out = torch.empty(world * width, local.shape[1], dtype=local.dtype, device=self.device)
+        dist.all_gather_into_tensor(out, buf)
+        blocks = []
+        for r in range(world):
+            lo, hi = self.shard_windows(n_windows, r, world)
+            blocks.append(out[r * width:r * width + hi - lo])
+        return torch.cat(blocks)
+
+    def _rank_world(self, rank, world):
+        if rank is None or world is None:
+            dist = torch.distributed
+            on = dist.is_available() and dist.is_initialized()
+            return (dist.get_rank(), dist.get_world_size()) if on else (0, 1)
+        return int(rank), int(world)
+
+    def validate(self, vset, chunk=64, rank=None, world=None):
+        """Held-out denoising loss of the current weights on `vset` (a `ValidationSet`): the per-sample loss of
+        `denoising_loss` for every (window, band) row at the band's timestep t_k and the window's fixed noise, `chunk`
+        rows per forward.  Windows are split by `shard_windows(W, rank, world)` (default: torch.distributed's rank and
+        world size); under a process group the per-window losses are all-gathered and every rank reduces them in window
+        order, otherwise the local block is returned.  Returns {"bands", "loss_by_band" (K,), "val_loss", "per_window"
+        (n, K), "windows" (lo, hi)}, float64 numpy; val_loss = mean_k loss_weight[t_k] loss_by_band[k], the training
+        objective (without the SIC term) under stratified t."""
+        rank, world = self._rank_world(rank, world)
+        W, bands = vset.windows, list(vset.bands)
+        K = len(bands)
+        lo, hi = self.shard_windows(W, rank, world)
+        rows = [(w, k) for w in range(lo, hi) for k in range(K)]
+        local = torch.zeros(hi - lo, K, dtype=torch.float64, device=self.device)
+        was_training = self.model.training
+        self.model.eval()
+        try:
+            for s in range(0, len(rows), int(chunk)):
+                rr = rows[s:s + int(chunk)]
+                wi = torch.tensor([w for w, _ in rr], device=self.device)
+                t = torch.tensor([bands[k] for _, k in rr], device=self.device)
+                loss = self.denoising_loss(vset.x0[wi], vset.cond[wi], vset.m1[wi], t, vset.noise[wi])
+                local.view(-1)[s:s + len(rr)] = loss
+        finally:
+            self.model.train(was_training)
+        per = self._gather_windows(local, W, rank, world).cpu().numpy()
+        by_band = per.mean(axis=0)
+        lw = self.loss_weight.detach().double().cpu().numpy()[bands]
+        return {"bands": bands, "loss_by_band": by_band, "val_loss": float(np.mean(lw * by_band)), "per_window": per,
+                "windows": (0, W) if per.shape[0] == W else (lo, hi)}
+
+    def score_samples(self, vset, sampler="dpm++2m", num_steps=20, seed=0, chunk=32, rank=None, world=None):
+        """Sample the validation mixtures of `vset` through `sample_windows` (window id = mixture index, x_T from
+        (seed, id)) and score every map against its clean map with `dq_map_scores`.  Sharding and gather as `validate`.
+        Returns {"per_window": {cosine, rmse, spectral_angle, xic_corr: (n,) arrays}, "mean": {the same: floats},
+        "windows": (lo, hi)}."""
+        from ..utils.validation import SCORE_KEYS, finalize_scores
+
+        rank, world = self._rank_world(rank, world)
+        W = vset.windows
+        lo, hi = self.shard_windows(W, rank, world)
+
+        def cond_fn(ids):
+            idx = torch.tensor(ids, device=self.device)
+            return vset.cond[idx], vset.m1[idx]
+
+        _, maps = self.sample_windows(range(W), cond_fn, seed=seed, num_steps=num_steps, chunk=chunk, rank=rank,
+                                      world=world, sampler=sampler)
+        local = torch.zeros(hi - lo, 9, dtype=torch.float64, device=self.device)
+        for s in range(0, hi - lo, int(chunk)):
+            e = min(hi - lo, s + int(chunk))
+            local[s:e] = self.map_scores(maps[s:e].to(self.device), vset.x0[lo + s:lo + e])
+        sums = self._gather_windows(local, W, rank, world)
+        sc = finalize_scores(sums, vset.x0.shape[1], vset.x0.shape[2])
+        per = {k: sc[k] for k in SCORE_KEYS}
+        return {"per_window": per, "mean": {k: float(np.mean(v)) for k, v in per.items()},
+                "windows": (0, W) if sums.shape[0] == W else (lo, hi)}
 
     def predict_windows(self, dataloader, mixture_weights=(0.5, 0.5), num_steps=50, seed=0, sampler="reference"):
         """`predict` for throughput: every batch item is kept and scored.  Returns a list of dicts

@@ -25,6 +25,8 @@ def load_train_config(config_path: str, **kwargs):
             cfg[sect][name] = kwargs[key]
     if kwargs.get("threads") is not None:
         cfg["threads"] = kwargs["threads"]
+    if kwargs.get("validation_fraction") is not None:   # optional section, absent from the default schema
+        cfg.setdefault("validation", {})["fraction"] = kwargs["validation_fraction"]
     return cfg
 
 

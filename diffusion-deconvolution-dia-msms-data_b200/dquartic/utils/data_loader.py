@@ -66,21 +66,38 @@ class DIAMSDataset(Dataset):
     def __len__(self):
         return len(self.ms2_data)
 
+    @property
+    def n_train(self):
+        """Training pairs are drawn from slices [0, n_train); the rest is held out for validation
+        (`dquartic.utils.validation.hold_out`).  Default: every slice."""
+        n = getattr(self, "_n_train", None)
+        return len(self.ms2_data) if n is None else n
+
+    @n_train.setter
+    def n_train(self, n):
+        if not 2 <= int(n) <= len(self.ms2_data):
+            raise ValueError(f"{n} training slices of {len(self.ms2_data)}: at least 2 are needed to draw a pair")
+        self._n_train = int(n)
+
     def draw_pair(self):
-        """The reference's rejection loop (data_loader.py:111-125): returns (idx_1, idx_2)."""
-        n = len(self.ms2_data)
+        """The reference's rejection loop (data_loader.py:111-125) over the training slices: returns (idx_1, idx_2)."""
+        return self.pair_from(random, 0, self.n_train, self.used_pairs)
+
+    def pair_from(self, rng, lo, hi, used):
+        """The rejection loop with the random source `rng` over slices [lo, hi), not repeating an unordered pair in (and
+        adding it to) `used`."""
         while True:
-            idx_1 = random.randint(0, n - 1)
-            idx_2 = random.randint(0, n - 1)
+            idx_1 = rng.randint(lo, hi - 1)
+            idx_2 = rng.randint(lo, hi - 1)
             if idx_1 == idx_2:
                 continue
             meta = getattr(self, "pair_meta", None)
             if meta is not None and meta[idx_1] == meta[idx_2]:
                 continue
             pair = tuple(sorted((idx_1, idx_2)))
-            if pair in self.used_pairs:
+            if pair in used:
                 continue
-            self.used_pairs.add(pair)
+            used.add(pair)
             return idx_1, idx_2
 
     def __getitem__(self, idx):
@@ -116,8 +133,8 @@ class DeviceBatchLoader:
         self.batch_size = int(batch_size)
         self.device = torch.device(device)
         self.pool = pool
-        n = len(dataset)
-        self.batches_per_epoch = batches_per_epoch or (n + self.batch_size - 1) // self.batch_size
+        n = len(dataset)   # the whole pool lives on the device, held-out slices included (validation mixtures)
+        self.batches_per_epoch = batches_per_epoch or (dataset.n_train + self.batch_size - 1) // self.batch_size
         ms2 = np.asarray(dataset.ms2_data)
         ms1 = np.asarray(dataset.ms1_data)
         if ms2.dtype in (np.int32, np.int64, np.int16, np.uint16, np.uint8, np.int8):

@@ -43,6 +43,13 @@ int dq_dpm_step(const float* xt, const float* model_out, float* d_hist, float* x
 int dq_scale_by(const float* x, const float* scale1, float* out, long n, void* stream);
 /* evaluation metric (model_interface.py:630-667 consumer): out3[s] += {<a_s, b_s>, |a_s|^2, |b_s|^2} per window s. */
 int dq_cosine_sums(const float* a, const float* b, float* out3, long n_per_sample, int n_samples, void* stream);
+/* validation scores of predicted maps against clean maps, both (n_windows, rt, mz) fp32: out9[w] = 9 float64 sums
+ * {sum (p-g)^2, sum pg, sum p^2, sum g^2, sum_mz PG, sum_mz P^2, sum_mz G^2, sum_mz w r, sum_mz w} with P, G the RT-summed
+ * spectra, r the Pearson correlation of a column over RT and w = G (0 for a truth column of zero variance).
+ * partial: n_windows * dq_map_scores_nblk(mz) * 9 doubles of scratch.  No atomics: bit-identical per window in any batch. */
+int dq_map_scores_nblk(int mz);
+int dq_map_scores(const float* pred, const float* truth, double* partial, double* out9, int n_windows, int rt, int mz,
+                  void* stream);
 /* tail of sample(): model.py:319-322. */
 int dq_sample_finalize(const float* x, const float* cond_n, float* xo, float* pn, long n, void* stream);
 /* sum (eps-noise)^2 into a double accumulator and d_eps = gscale*(eps-noise): F.mse_loss model.py:361. */

@@ -43,4 +43,25 @@ p, ms2 = np.load("pred.npy"), np.load("ms2.npy")
 print("predicted", p.shape, p.dtype, "range", float(p.min()), float(p.max()))
 assert p.shape == ms2.shape and p.dtype == np.float32 and np.isfinite(p).all()
 PY
+# hold out 25 % of the pool (6 slices: 15 pairs), select the best checkpoint by the EMA's validation loss, then score it
+mkdir -p ckpt_val
+python - <<'PY'
+import json
+c = json.load(open("cfg.json"))
+c["validation"] = {"fraction": 0.25, "windows": 12, "bands": 5, "seed": 3}
+json.dump(c, open("cfg_val.json", "w"), indent=1)
+PY
+python -m dquartic.cli train --ms2-data-path ms2.npy --ms1-data-path ms1.npy --checkpoint-path ckpt_val/best_model.ckpt \
+    --ema-decay 0.99 cfg_val.json 2>&1 | grep -E "Validation|Best model"
+python -m dquartic.cli evaluate --checkpoint-path ckpt_val/best_model.ckpt --ms2-data-path ms2.npy --ms1-data-path ms1.npy \
+    --weights both --num-steps 10 --chunk 4 --output eval.json cfg_val.json
+python - <<'PY'
+import json, math, torch
+r = json.load(open("eval.json"))
+ck = torch.load("ckpt_val/best_model.ckpt", map_location="cpu", weights_only=False)
+print("evaluate:", {w: (v["val_loss"], v["samplers"]["dpm++2m@10"]["mean"]) for w, v in r["results"].items()})
+assert r["windows"] == 12 and r["results"]["ema"]["val_loss"] == ck["val_loss"] == ck["best_loss"]
+assert all(math.isfinite(x) for v in r["results"].values() for l in v["samplers"]["dpm++2m@10"]["per_window"].values()
+           for x in l)
+PY
 echo CLI_SMOKE_OK
