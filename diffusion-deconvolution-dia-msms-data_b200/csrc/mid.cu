@@ -511,6 +511,7 @@ using namespace dq;
 DQ_API int dq_mid_pack(const float* x, void* out_bf16, int b, int rt, int N, int pad, void* stream) {
   if (b <= 0) return 0;
   if (N & 1) return -3;
+  if (((size_t)x & 7) || ((size_t)out_bf16 & 3)) return -4;   // float2 loads, bf16x2 stores
   int rows = b * (pad ? rt + 2 : rt);
   mid_pack_kernel<<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>(x, (__nv_bfloat16*)out_bf16, b, rt, N, pad);
   DQ_LAUNCH_CHECK();
@@ -581,10 +582,18 @@ DQ_API int dq_rownorm_bwd(const float* dh, int dhpad, const float* u, int upad, 
   DQ_LAUNCH_CHECK();
   return 0;
 }
+// opt-in maximum of dynamic shared memory per block on the current device (227 KB on sm_100a)
+static size_t attn_smem_limit() {
+  int dev = 0, v = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  return (size_t)v;
+}
 DQ_API int dq_attn_core_fwd(const float* qv, const float* k, const float* freqs, float* P, float* o_f32, void* o_bf16,
                             int b, int rt, void* stream) {
   if (b <= 0) return 0;
   size_t smem = sizeof(float) * (3 * rt * 33 + rt * rt);
+  if (smem > attn_smem_limit()) return -2;   // rt too long for one CTA's shared memory
   cudaFuncSetAttribute(attn_core_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   attn_core_fwd_kernel<<<(unsigned)(b * 4), 128, smem, (cudaStream_t)stream>>>(qv, k, freqs, P, o_f32, (__nv_bfloat16*)o_bf16, rt);
   DQ_LAUNCH_CHECK();
@@ -594,6 +603,7 @@ DQ_API int dq_attn_core_bwd(const float* qv, const float* k, const float* freqs,
                             float* dqv, void* dqv_bf16, float* dk, int b, int rt, void* stream) {
   if (b <= 0) return 0;
   size_t smem = sizeof(float) * (4 * rt * 33 + 2 * rt * rt);
+  if (smem > attn_smem_limit()) return -2;
   cudaFuncSetAttribute(attn_core_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   attn_core_bwd_kernel<<<(unsigned)(b * 4), 128, smem, (cudaStream_t)stream>>>(qv, k, freqs, P, dO, dqv, (__nv_bfloat16*)dqv_bf16, dk, rt);
   DQ_LAUNCH_CHECK();

@@ -158,6 +158,7 @@ int dq_gemm_bf16_tn(const void* A, long a_rows, long a_cols, long a_ld, const vo
                     int M, int N, int K, int taps, const int* offs, int nz, int z_b_koff_step, int z_b_tap_step,
                     long z_c_stride, int bn, void* stream);
 int dq_gemm_last_error(void);
+/* -3: N odd; -4: x not 8-byte or out_bf16 not 4-byte aligned. */
 int dq_mid_pack(const float* x, void* out_bf16, int b, int rt, int N, int pad, void* stream);
 int dq_transpose_bf16(const void* in, void* out, int rows, int cols, long ld_out, int row_shift, void* stream);
 int dq_cast_transpose(const float* in, void* out_bf16, void* out_t_bf16, int rows, int cols, void* stream);
@@ -167,6 +168,7 @@ int dq_rownorm_bwd(const float* dh, int dhpad, const float* u, int upad, const f
                    int act, const float* inv, float* dot, void* du_bf16, int opad, float* du_f32, int du_acc, float* dg,
                    float* dss, float* dbias, int b, int rt, int N, void* stream);
 int dq_colsum(const float* x, float* out, int rows, int cols, void* stream);
+/* -2 (before any launch): the rt x rt tiles of one (sample, head) exceed the device's opt-in shared memory (sm_100a: rt > 196 forward, rt > 140 backward). */
 int dq_attn_core_fwd(const float* qv, const float* k, const float* freqs, float* P, float* o_f32, void* o_bf16, int b,
                      int rt, void* stream);
 int dq_attn_core_bwd(const float* qv, const float* k, const float* freqs, const float* P, const float* dO, float* dqv,

@@ -167,7 +167,7 @@ def rope(t, freqs):
     positions 0..n-1, angles pos*freqs repeated pairwise, interleaved-pair rotation of the first
     2*len(freqs) features, the rest pass through.  Call sites: model/unet1d.py:560-561."""
     n = t.shape[-2]
-    ang = torch.arange(n, dtype=torch.float32)[:, None] * freqs[None, :]  # (n, 8)
+    ang = torch.arange(n, dtype=torch.float32, device=t.device)[:, None] * freqs[None, :]  # (n, 8)
     ang = ang.repeat_interleave(2, dim=-1)  # (n, 16)
     rd = ang.shape[-1]
     tr, tp = t[..., :rd], t[..., rd:]
