@@ -10,7 +10,6 @@
 // Layout: activations fp32 (R, C, L) channel-planar (the reference's NCL), R = batch*RT rows.  A thread owns
 // all output channels of P positions (needed for the channel RMSNorm) that are blockDim apart, so every
 // global access is a coalesced 128-byte line per warp; the K taps hit the same lines in L1.
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace dq {
@@ -436,15 +435,13 @@ DQ_API int dq_conv1d_fwd(const float* x1, int c1, const float* x2, int c2, const
                 in_ss_stride, act};
   cudaStream_t st = (cudaStream_t)stream;
   if (R <= 0 || Lout <= 0) return 0;
-  static int new_modes = -1;   // DQ_CONV_FWD_K7_DN=0: init_conv / Downsample through the plain-load kernel (A/B runs)
-  if (new_modes < 0) { const char* e = getenv("DQ_CONV_FWD_K7_DN"); new_modes = (e && e[0] == '0') ? 0 : 1; }
-  if (stride == 1 && (!in_ss || K == 7) && (K != 7 || new_modes) && pad == (K - 1) / 2 && ((up == 1 && Lin == Lout) || (up == 2 && 2 * Lin == Lout))) {
+  if (stride == 1 && (!in_ss || K == 7) && pad == (K - 1) / 2 && ((up == 1 && Lin == Lout) || (up == 2 && 2 * Lin == Lout))) {
     // bulk-copy pipelined kernel (conv_fused.cu)
     int rc = conv_fwd_tma_try(x1, c1, x2, c2, w, bias, cout, K, g, ss, ss_stride, act, res, u, y, R, Lout, rows_per_sample, up, st,
                               in_ss, in_ss_stride);
     if (rc != 0) return rc < 0 ? rc : 0;
   }
-  if (new_modes && stride == 2 && K == 4 && pad == 1 && up == 1 && !in_ss && !x2 && !res && Lin == 2 * Lout) {
+  if (stride == 2 && K == 4 && pad == 1 && up == 1 && !in_ss && !x2 && !res && Lin == 2 * Lout) {
     // Downsample (unet1d.py:110) through the same pipelined kernel (up = -2: stride-2 mode)
     int rc = conv_fwd_tma_try(x1, c1, nullptr, 0, w, bias, cout, K, g, ss, ss_stride, act, nullptr, u, y, R, Lout, rows_per_sample, -2, st);
     if (rc != 0) return rc < 0 ? rc : 0;

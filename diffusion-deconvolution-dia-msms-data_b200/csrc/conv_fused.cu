@@ -15,7 +15,6 @@
 //            CTA lifetime, streaming du / x rows with 128-bit shared loads
 // and the parameter gradients leave the CTA once (shared-memory combine, then one global atomic per value).
 // HBM-bound: algorithmic bytes per position = 4 * (2 * COUT + 2 * cin) (+ 4 * c1 with dadd / accumulate).
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace dq {
@@ -1285,18 +1284,13 @@ static int dispatch_fused(const ConvBwdFusedArgs& a, int cout, cudaStream_t st) 
   const bool v4 = (a.L % 4 == 0);
   // 16-byte aligned rows: bulk-async-copy pipeline
   const bool al = v4 && ((((size_t)a.dy | (size_t)a.x1 | (size_t)a.u | (size_t)a.x2) & 15) == 0);
-  static int mode = -1;   // DQ_CONV_BWD_NOTMA=1 forces the plain-load kernels (cross-check)
-  if (mode < 0) { const char* e = getenv("DQ_CONV_BWD_NOTMA"); mode = (e && e[0] == '1') ? 1 : 0; }
   // the pipelined kernel covers: plain conv, or RMSNorm (+ scale/shift) + SiLU epilogue; channel counts in fours
   const bool epi_ok = !a.u || (a.g && a.act == 1);
   const int cin = a.c1 + a.c2;
-  static int mma_mode = -1;   // DQ_CONV_BWD_MMA=0: FFMA contractions everywhere (cross-check)
-  if (mma_mode < 0) { const char* e = getenv("DQ_CONV_BWD_MMA"); mma_mode = (e && e[0] == '0') ? 0 : 1; }
-  const bool mma_on = mma_mode == 1;
   const bool ch4 = (a.c1 & 3) == 0 && (a.c2 & 3) == 0;
   if constexpr (K == 3) {
     // conv3 + RMSNorm / SiLU epilogue at 8 .. 16 channels: tensor-core contractions (NCI = n8 tiles over cin)
-    if (mode == 0 && mma_on && !a.dyo && a.L >= 128 && a.u && a.g && a.act == 1 && ch4 && cin <= 32) {
+    if (!a.dyo && a.L >= 128 && a.u && a.g && a.act == 1 && ch4 && cin <= 32) {
       const int nci = (cin + 7) / 8;
       if (al) {
         if (cout == 8 && nci == 1) return launch_fused_tma<8, 3, 2, 128, true, true, false, 1>(a, st);
@@ -1312,18 +1306,18 @@ static int dispatch_fused(const ConvBwdFusedArgs& a, int cout, cudaStream_t st) 
   if (a.dyo) {   // conv3 + epilogue with the 1x1 res_conv over the same input: pipelined kernel only
     if constexpr (K == 3) {
       const bool al2 = al && (((size_t)a.dyo & 15) == 0);
-      if (mode == 0 && a.L >= 128 && a.u && a.g && a.act == 1 && ch4 && !a.dadd) {
+      if (a.L >= 128 && a.u && a.g && a.act == 1 && ch4 && !a.dadd) {
         const int nci = (cin + 7) / 8;
         if (al2) {
           if (cout == 4) return launch_fused_tma<4, 3, 4, 128, true, true, true>(a, st);
           if (cout == 8) {
-            if (mma_on && nci == 1) return launch_fused_tma<8, 3, 2, 128, true, true, true, 1>(a, st);
-            if (mma_on && nci == 2) return launch_fused_tma<8, 3, 2, 128, true, true, true, 2>(a, st);
+            if (nci == 1) return launch_fused_tma<8, 3, 2, 128, true, true, true, 1>(a, st);
+            if (nci == 2) return launch_fused_tma<8, 3, 2, 128, true, true, true, 2>(a, st);
             return launch_fused_tma<8, 3, 2, 128, true, true, true>(a, st);
           }
-          if (mma_on && cout == 12 && nci == 3) return launch_fused_tma<12, 3, 1, 128, true, true, true, 3>(a, st);
-          if (mma_on && cout == 16 && nci == 4) return launch_fused_tma<16, 3, 1, 128, true, true, true, 4>(a, st);
-        } else if (mma_on) {
+          if (cout == 12 && nci == 3) return launch_fused_tma<12, 3, 1, 128, true, true, true, 3>(a, st);
+          if (cout == 16 && nci == 4) return launch_fused_tma<16, 3, 1, 128, true, true, true, 4>(a, st);
+        } else {
           if (cout == 12 && nci == 3) return launch_fused_tma<12, 3, 1, 128, true, false, true, 3>(a, st);
           if (cout == 16 && nci == 4) return launch_fused_tma<16, 3, 1, 128, true, false, true, 4>(a, st);
         }
@@ -1331,7 +1325,7 @@ static int dispatch_fused(const ConvBwdFusedArgs& a, int cout, cudaStream_t st) 
     }
     return 1;    // not covered: the caller runs the two convolutions separately
   }
-  if (mode == 0 && a.L >= 128 && epi_ok && (a.c1 & 3) == 0 && (a.c2 & 3) == 0) {
+  if (a.L >= 128 && epi_ok && ch4) {
     if (al) {
       switch (cout) {
         case 4: return launch_fused_tma_epi<4, K, 4, 128, true>(a, st);
@@ -1643,9 +1637,7 @@ static int launch_fwd_tma(ConvFwdTmaArgs a, cudaStream_t st) {
 int conv_fwd_tma_try(const float* x1, int c1, const float* x2, int c2, const float* w, const float* bias, int cout, int K,
                      const float* g, const float* ss, int ss_stride, int act, const float* res, float* u, float* y, int R,
                      int L, int rows_per_sample, int up, cudaStream_t st, const float* in_ss, int in_ss_stride) {
-  static int mode = -1;   // DQ_CONV_FWD_NOTMA=1 forces the plain-load kernel (cross-check)
-  if (mode < 0) { const char* e = getenv("DQ_CONV_FWD_NOTMA"); mode = (e && e[0] == '1') ? 1 : 0; }
-  if (mode == 1 || L < 128 || c1 + c2 > 64) return 0;
+  if (L < 128 || c1 + c2 > 64) return 0;
   if (up == -2) { if (K != 4 || x2 || res) return 0; }   // Downsample: k4, stride 2, pad 1; L = output length
   else if (K == 7) { if (up != 1 || res || (cout != 4 && cout != 8)) return 0; }
   else if (K != 1 && K != 3) return 0;
@@ -2427,15 +2419,10 @@ DQ_API int dq_resblock_fwd(const float* x1, int c1, const float* x2, int c2, con
   if (R <= 0 || L <= 0) return 0;
   const int cin = c1 + c2;
   if (L < 128 || cin > 32 || (cin & 3) || (c1 & 3) || (!wres && cin != cout)) return 1;
-  static int mode = -1;   // DQ_RESBLOCK_FUSED=0: compose from single-conv kernels (cross-check)
-  if (mode < 0) { const char* e = getenv("DQ_RESBLOCK_FUSED"); mode = (e && e[0] == '0') ? 0 : 1; }
-  if (!mode) return 1;
   ResFwdArgs a{x1, x2, w1, b1, g1, ss, w2, b2, g2, wres, bres, u1, h1, u2, out, c1, c2, R, L, rows_per_sample, ss_stride, 0, 0, 0};
   const bool al = (L % 4 == 0) && ((((size_t)x1 | (size_t)x2 | (size_t)u1 | (size_t)h1 | (size_t)u2 | (size_t)out) & 15) == 0);
   cudaStream_t st = (cudaStream_t)stream;
-  static int mma_mode = -1;   // DQ_RESBLOCK_MMA=0: FFMA kernels at every channel count (cross-check)
-  if (mma_mode < 0) { const char* e = getenv("DQ_RESBLOCK_MMA"); mma_mode = (e && e[0] == '0') ? 0 : 1; }
-  if (mma_mode && cout >= 8) {
+  if (cout >= 8) {
     const int kci = (cin + 7) / 8;
     if (al) {
       // (cout 8, cin 8: the FFMA2 kernel is as fast — 6 warp-instructions per position of conv work either way)

@@ -12,12 +12,18 @@
 // Replaces (reference /root/reference/dquartic/model/unet1d.py): the four Conv1d(10000,10000,3,padding=1)
 // of mid_block1/2 (243, 1029, 1058) forward / dgrad / wgrad, and Attention.to_qv / to_out 1x1 convs (534, 539).
 //
-// Structure: one 128 x BN output tile per CTA, 192 threads = warp 0 TMA producer, warp 1 MMA issuer (+ TMEM
+// Structure: a persistent kernel, one CTA per SM, 192 threads = warp 0 TMA producer, warp 1 MMA issuer (+ TMEM
 // alloc), warps 2-5 epilogue (TMEM lane quadrant = warp_idx % 4).  STAGES-deep smem ring of 128B-swizzled
 // [128|BN] x 64 bf16 tiles filled by cp.async.bulk.tensor, consumed by tcgen05.mma.cta_group::1.kind::f16
 // (M=128, N=BN, K=16) with fp32 accumulators in TMEM; tcgen05.commit releases ring slots / signals the epilogue.
+//   * each CTA walks a static round-robin list of 128 x BN output tiles; the smem operand ring keeps running across
+//     tiles
+//   * two TMEM accumulator buffers: the epilogue warps drain tile i while the MMA warp already accumulates tile i+1
+//   * tile width BN is a RUN-TIME multiple of 16 (<= 256) picked by the host so that tiles / #SMs has no ragged last wave
+//     (M = 1152, N = 10000: 128 x 208 tiles -> 441 tiles = 2.98 waves instead of 360 tiles = 2.43 -> 3 waves at BN 256)
+//   * tiles are rasterised in GM x GN super-tiles so that the operands of one wave fit the 126 MB L2 (the K = 9216 weight
+//     gradient re-read its operands 26x from DRAM with the plain m-fastest order)
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 #include "common.cuh"
 
@@ -120,131 +126,7 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-template <int BN, int STAGES>
-__global__ void __launch_bounds__(192, 1)
-gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, GemmParams p) {
-  constexpr uint32_t A_BYTES = BM * BK * 2, B_BYTES = BN * BK * 2, STAGE_BYTES = A_BYTES + B_BYTES;
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen_base = smem_raw + (sbase - smem_u32(smem_raw));
-  const uint32_t bars = sbase + STAGES * STAGE_BYTES;  // full[STAGES], empty[STAGES], tmem_full, then tmem ptr
-  const uint32_t full0 = bars, empty0 = bars + 8 * STAGES, tfull = bars + 16 * STAGES;
-  volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(gen_base + STAGES * STAGE_BYTES + 16 * STAGES + 8);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m_tile = blockIdx.x % p.m_tiles, n_tile = blockIdx.x / p.m_tiles, z = blockIdx.y;
-  const int m0 = m_tile * BM, n0 = n_tile * BN;
-  const int kblocks = (p.K + BK - 1) / BK;
-  const int iters = kblocks * p.taps;
-
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < STAGES; ++s) {
-        mbar_init(full0 + 8 * s, 1);
-        mbar_init(empty0 + 8 * s, 1);
-      }
-      mbar_init(tfull, 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_slot)), "r"((uint32_t)BN) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_d = *tmem_slot;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      int s = 0;
-      uint32_t ph = 0;
-      for (int it = 0; it < iters; ++it) {
-        const int tap = it / kblocks, kb = it - tap * kblocks;
-        mbar_wait(empty0 + 8 * s, ph ^ 1, p.err, 1);
-        mbar_expect_tx(full0 + 8 * s, STAGE_BYTES);
-        const uint32_t sa = sbase + s * STAGE_BYTES, sb = sa + A_BYTES;
-        tma_load_2d(sa, &tmA, full0 + 8 * s, kb * BK + p.a_k_off[tap], m0 + p.a_row_off[tap]);
-        tma_load_3d(sb, &tmB, full0 + 8 * s, kb * BK + p.b_k_off[tap] + z * p.z_b_koff_step, n0, p.b_tap[tap] + z * p.z_b_tap_step);
-        if (++s == STAGES) { s = 0; ph ^= 1; }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      // instruction descriptor: D=f32, A=B=bf16, both K-major, N=BN, M=128
-      constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-      int s = 0;
-      uint32_t ph = 0;
-      for (int it = 0; it < iters; ++it) {
-        mbar_wait(full0 + 8 * s, ph, p.err, 2);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint32_t sa = sbase + s * STAGE_BYTES, sb = sa + A_BYTES;
-#pragma unroll
-        for (int k = 0; k < BK / 16; ++k) {
-          umma_bf16(tmem_d, umma_desc_sw128(sa + k * 32), umma_desc_sw128(sb + k * 32), idesc, (it > 0 || k > 0) ? 1u : 0u);
-        }
-        umma_commit(empty0 + 8 * s);  // frees the smem slot once these MMAs have read it
-        if (++s == STAGES) { s = 0; ph ^= 1; }
-      }
-      umma_commit(tfull);  // accumulator complete
-    }
-  } else {
-    // epilogue: warps 2..5 -> TMEM lane quadrant warp % 4
-    mbar_wait(tfull, 0, p.err, 3);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const int q = warp & 3;
-    const int row = m0 + q * 32 + lane;
-    float* crow = p.C + (size_t)z * p.z_c_stride + (size_t)row * p.ldc;
-    const bool vec_ok = ((p.ldc & 3) == 0) && ((((size_t)(p.C + (size_t)z * p.z_c_stride)) & 15) == 0);
-#pragma unroll 1
-    for (int c = 0; c < BN / 32; ++c) {
-      uint32_t r[32];
-      tmem_ld32(tmem_d + ((uint32_t)(q * 32) << 16) + (uint32_t)(c * 32), r);
-      if (row < p.M) {
-        const int nb = n0 + c * 32;
-#pragma unroll
-        for (int i = 0; i < 32; i += 4) {
-          const int n = nb + i;
-          if (n >= p.N) break;
-          float v0 = __uint_as_float(r[i]), v1 = __uint_as_float(r[i + 1]), v2 = __uint_as_float(r[i + 2]), v3 = __uint_as_float(r[i + 3]);
-          if (vec_ok && n + 3 < p.N) {
-            if (p.bias) {
-              float4 b4 = *reinterpret_cast<const float4*>(p.bias + n);
-              v0 += b4.x; v1 += b4.y; v2 += b4.z; v3 += b4.w;
-            }
-            float4* dst = reinterpret_cast<float4*>(crow + n);
-            if (p.accumulate) {
-              float4 o = *dst;
-              v0 += o.x; v1 += o.y; v2 += o.z; v3 += o.w;
-            }
-            *dst = make_float4(v0, v1, v2, v3);
-          } else {
-            float vv[4] = {v0, v1, v2, v3};
-            for (int t = 0; t < 4 && n + t < p.N; ++t) {
-              float v = vv[t] + (p.bias ? p.bias[n + t] : 0.f);
-              if (p.accumulate) v += crow[n + t];
-              crow[n + t] = v;
-            }
-          }
-        }
-      }
-    }
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"((uint32_t)BN) : "memory");
-  }
-}
-
-// =====================================================================================================================
-// v2: persistent, epilogue-overlapped variant.
-//   * one CTA per SM walks a static round-robin list of output tiles; the smem operand ring keeps running across tiles
-//   * two TMEM accumulator buffers: the epilogue warps drain tile i while the MMA warp already accumulates tile i+1
-//   * tile width BN is a RUN-TIME multiple of 16 (<= 256) picked by the host so that tiles / #SMs has no ragged last wave
-//     (M = 1152, N = 10000: 128 x 208 tiles -> 441 tiles = 2.98 waves instead of 360 tiles = 2.43 -> 3 waves at BN 256)
-//   * tiles are rasterised in GM x GN super-tiles so that the operands of one wave fit the 126 MB L2 (the K = 9216 weight
-//     gradient re-read its operands 26x from DRAM with the plain m-fastest order)
+// the problem (GemmParams) plus the run-time tile width, ring depth and tile-walk geometry
 struct GemmParams2 {
   GemmParams g;
   int bn, stages, tiles_m, tiles_n, nz, gm, gn;
@@ -450,20 +332,6 @@ static EncodeTiledFn get_encode() {
 }
 
 static unsigned long long* g_err_flag = nullptr;
-
-template <int BN, int STAGES>
-static int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, GemmParams p, int nz, cudaStream_t st) {
-  constexpr size_t smem = (size_t)STAGES * (BM * BK * 2 + BN * BK * 2) + 16 * STAGES + 16 + 1024;
-  auto kern = gemm_tcgen05_kernel<BN, STAGES>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  int n_tiles = (p.N + BN - 1) / BN;
-  dim3 grid((unsigned)(p.m_tiles * n_tiles), (unsigned)nz);
-  kern<<<grid, 192, smem, st>>>(tmA, tmB, p);
-  DQ_LAUNCH_CHECK();
-  return 0;
-}
-
 static int g_sm_count = 0;
 
 // tile width that minimises (waves x tile cost): no ragged last wave; ties go to the wider tile (less L2 traffic)
@@ -481,7 +349,7 @@ static int pick_bn(int m_tiles, int N, int nz, int sms) {
   return best;
 }
 
-static int launch_gemm_v2(const CUtensorMap& tmA, const CUtensorMap& tmB, GemmParams p, int nz, int bn, cudaStream_t st) {
+static int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, GemmParams p, int nz, int bn, cudaStream_t st) {
   GemmParams2 pp;
   pp.g = p;
   pp.bn = bn;
@@ -512,7 +380,8 @@ using namespace dq;
 
 // A: bf16 (a_rows, a_cols) with leading dimension a_ld (elements); B: bf16 (b_ntaps, b_rows, b_cols) with
 // row stride b_ld and tap stride b_tap_stride (elements).  All strides must be multiples of 8 elements (16 B).
-// offs: 16 ints = a_row_off[4], a_k_off[4], b_k_off[4], b_tap[4].
+// offs: 16 ints = a_row_off[4], a_k_off[4], b_k_off[4], b_tap[4].  bn: tile width, a multiple of 16 up to 256;
+// any other value lets pick_bn choose it.
 DQ_API int dq_gemm_bf16_tn(const void* A, long a_rows, long a_cols, long a_ld, const void* B, long b_rows, long b_cols,
                            long b_ld, long b_tap_stride, int b_ntaps, float* C, long ldc, const float* bias,
                            int accumulate, int M, int N, int K, int taps, const int* offs, int nz, int z_b_koff_step,
@@ -527,11 +396,8 @@ DQ_API int dq_gemm_bf16_tn(const void* A, long a_rows, long a_cols, long a_ld, c
     cudaMemset(g_err_flag, 0, sizeof(unsigned long long));
   }
   if (!g_sm_count) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&g_sm_count, cudaDevAttrMultiProcessorCount, dev); }
-  static int v1 = -1;   // DQ_GEMM_V1=1: the one-tile-per-CTA kernel (cross-check)
-  if (v1 < 0) { const char* e = getenv("DQ_GEMM_V1"); v1 = (e && e[0] == '1') ? 1 : 0; }
-  const int m_tiles_h = (M + BM - 1) / BM;
-  if (v1) { if (bn != 256) bn = 128; }
-  else if (bn <= 0 || bn % 16 || bn > 256) bn = pick_bn(m_tiles_h, N, nz < 1 ? 1 : nz, g_sm_count);
+  if (nz < 1) nz = 1;
+  if (bn <= 0 || bn % 16 || bn > 256) bn = pick_bn((M + BM - 1) / BM, N, nz, g_sm_count);
   CUtensorMap tmA, tmB;
   {
     cuuint64_t dims[2] = {(cuuint64_t)a_cols, (cuuint64_t)a_rows};
@@ -563,9 +429,7 @@ DQ_API int dq_gemm_bf16_tn(const void* A, long a_rows, long a_cols, long a_ld, c
   if (z_b_koff_step % 8) return -4;
   p.z_b_koff_step = z_b_koff_step; p.z_b_tap_step = z_b_tap_step; p.accumulate = accumulate; p.m_tiles = (M + BM - 1) / BM; p.err = g_err_flag;
   cudaStream_t st = (cudaStream_t)stream;
-  if (!v1) return launch_gemm_v2(tmA, tmB, p, nz < 1 ? 1 : nz, bn, st);
-  if (bn == 256) return launch_gemm<256, 4>(tmA, tmB, p, nz < 1 ? 1 : nz, st);
-  return launch_gemm<128, 6>(tmA, tmB, p, nz < 1 ? 1 : nz, st);
+  return launch_gemm(tmA, tmB, p, nz, bn, st);
 }
 
 // reads (and clears) the pipeline-timeout flag: 0 = ok, 1 = producer, 2 = MMA, 3 = epilogue wait timed out

@@ -1189,16 +1189,13 @@ template <int C>
 static int la_bwd(const LAArgs& a, cudaStream_t st) {
   using T = TC<C>;
   dim3 grid((unsigned)a.nchunk, (unsigned)a.R);
-  bool q_done = false;
   // tcgen05 / TMEM kernel (linattn_tc.cu) where it wins: per launch of a 64-sample micro-batch 9.43 -> 5.89 ms (C = 4),
   // 3.95 -> 3.24 (C = 8), 1.82 -> 1.18 (C = 12); at C = 16 (L <= 1250: 5-10 tiles per CTA, fixed cost dominates, spills) it
   // measured 1.21 vs 0.71 ms, so the mma.sync kernel keeps that level (profiles/r2_launches_summary.csv vs r1d)
   if (la_tc_enabled() && C <= 12) {
     const int rc = la_bwd_q_tc(a, C, st);
     if (rc != 0) return rc;
-    q_done = true;
-  }
-  if (!q_done) {
+  } else {
     size_t smem = sizeof(float) * ((C == 4 ? 1 : 2) * TA<C>::SIZE + 2 * C * XT + 4 * SP * T::YS + 4 * 2 * 16 * RS + 2 * C +
                                    (C == 4 ? 3 * C * SP : 0));
     cudaFuncSetAttribute(la_bwd_q_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1212,11 +1209,6 @@ static int la_bwd(const LAArgs& a, cudaStream_t st) {
     la_bwd_combine_kernel<C><<<(unsigned)((a.R + kRows - 1) / kRows), 128, smem, st>>>(a, kRows);
     DQ_LAUNCH_CHECK();
   }
-  // DQ_LA_KV_TC=1 selects the hybrid tcgen05-scores + mma.sync-f16 k / v kernel (linattn_tc.cu).  Measured slower than
-  // the mma.sync kernel below (level 0, 8 samples: 0.93 vs 0.81 ms, profiles/r2_la_bwd_kv_tc_*), so it stays opt-in.
-  static int kv_tc = -1;
-  if (kv_tc < 0) { const char* e = getenv("DQ_LA_KV_TC"); kv_tc = (e && e[0] == '1') ? 1 : 0; }
-  if (la_tc_enabled() && kv_tc && (C == 4 || C == 8)) return la_bwd_kv_tc(a, C, st);   // hybrid tcgen05 + mma.sync f16 kernel
   {
     size_t smem = sizeof(float) * (TA<C>::SIZE + C * XT + 4 * SP * T::YS + 4 * 16 * RS + SP + C + (C <= LA_KV_ASYNC_MAXC ? 4 * C * SP : 0));
     cudaFuncSetAttribute(la_bwd_kv_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

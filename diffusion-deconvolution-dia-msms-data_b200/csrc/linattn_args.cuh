@@ -32,7 +32,6 @@ struct LAArgs {
 };
 
 // tcgen05 / TMEM kernels (linattn_tc.cu).  Return 0 on launch, -3 when the channel count is not covered.
-int la_bwd_q_tc(const LAArgs& a, int C, cudaStream_t st);
-int la_bwd_kv_tc(const LAArgs& a, int C, cudaStream_t st);   // C = 4, 8
+int la_bwd_q_tc(const LAArgs& a, int C, cudaStream_t st);   // C = 4, 8, 12
 
 }  // namespace dq

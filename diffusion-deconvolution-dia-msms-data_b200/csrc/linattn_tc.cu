@@ -21,7 +21,6 @@
 // staging warps and keeping tcgen05 for the N = 256 score product only is the next step (DESIGN.md).
 #include <stdio.h>
 #include <stdlib.h>
-#include <cuda_fp16.h>
 #include "linattn_args.cuh"
 #include "linattn_tc.cuh"
 
@@ -454,387 +453,6 @@ static int launch_bwd_q(const LAArgs& a, cudaStream_t st) {
   return 0;
 }
 
-
-// =====================================================================================================================
-// backward, k / v path (hybrid).  Per row r and chunk of positions (notation of linattn.cu):
-//   ks = softmax_L(k) = 2^(log2e k + cn),  dks = H xn - sd,  dk = ks dks,
-//   d xn = Wk^T dk + H^T ks (+ d xn_q), RMSNorm_pre backward, + dres -> dx;   dWk += dk^T xn;   d g_pre.
-// tcgen05 does the one product whose N is large - the scores [128 positions x (128 k' | 128 dks')] = Xn [128 x K] . B^T,
-// two MMAs per tile into a TMEM slot of 256 columns, constants (cn, -sd) riding in two spare K slots of the operand.
-// A thread owns a position and a head: 32 exponentials + 32 multiplies, results as f16 [d][pos] tiles in shared memory.
-// The products with 8 output columns (d xn: contraction over (head, d); dWk: contraction over positions) run as
-// ldmatrix + mma.sync m16n8k16 on four "reduce" warps, which also do the epilogue of their 32 positions.
-// f16 needs a known scale: ks' = 2^11 ks <= 2048; H' = 2^e H with e from a per-row bound such that |dks'| <= 1; so
-// dk' = ks' dks' = 2^(11 + e) dk; every accumulator is multiplied by 2^-(11 + e) once.  f16 has TF32's mantissa.
-template <int C>
-struct BK {
-  static constexpr int CL = (C + 7) / 8 * 8;              // padded channel count of the saved statistics (msm, hmat)
-  static constexpr int CP = (C + 2 + 7) / 8 * 8;          // K of the score products: channels + 2 constant slots
-  static constexpr int KS = CP / 8;
-  static constexpr uint32_t A_SBO = 128 * (CP / 4);
-  static constexpr int A_BYTES = 128 * CP * 4;
-  static constexpr int NSTG = 3;
-  static constexpr int XT_ROW = 272;                      // bytes per row of the f16 xn^T stage (68 words: conflict-free B loads)
-  static constexpr int XT_BYTES = 8 * XT_ROW;
-  static constexpr int XS_BYTES = C * 128 * 4;            // raw x [c][pos] for the epilogue
-  static constexpr int TILE = 128 * 128 * 2;              // f16 [16 d-groups][128 pos][8]
-  static constexpr int oBK = 0;                           // [128 (h, d) x CP] tf32: log2e Wk | cn_hi | cn_lo
-  static constexpr int oBH = oBK + A_BYTES;               // [128 x CP] tf32: H' | -sd'_hi | -sd'_lo
-  static constexpr int oAX = oBH + A_BYTES;               // NSTG x [128 pos x CP] tf32: xn | 1 | 1
-  static constexpr int oXT = oAX + NSTG * A_BYTES;        // NSTG x f16 xn^T [8][128 (+pad)]
-  static constexpr int oXS = oXT + NSTG * XT_BYTES;       // NSTG x raw x
-  static constexpr int oINV = oXS + NSTG * XS_BYTES;      // NSTG x 1 / |x|
-  static constexpr int oKS = oINV + NSTG * 512;           // 2 x ks' tile
-  static constexpr int oDK = oKS + 2 * TILE;              // 2 x dk' tile
-  static constexpr int oDXN = oDK + 2 * TILE;             // [128 pos][8] fp32: d xn of the tile being finished
-  static constexpr int oPF = oDXN + 128 * 8 * 4;           // [2][C][128] fp32: dxn_q | dres of the tile being finished (cp.async)
-  static constexpr int oBAR = oPF + 2 * C * 128 * 4;
-  static constexpr int NBAR = 24;
-  static constexpr int SMEM = oBAR + NBAR * 8 + 32 + 128;
-};
-constexpr int kThreadsK = 25 * 32;   // 16 compute + 4 staging (+ dWk) + 4 reduce / epilogue + 1 MMA-issuing warp
-constexpr int kS = 0, kLD = 2, kTILE = 4, kTFREE = 6, kFULL = 8, kSFREE = 11;
-
-template <int C>
-__global__ void __launch_bounds__(kThreadsK, 1) la_bwd_kv_tc_kernel(LAArgs a) {
-  using K = BK<C>;
-  extern __shared__ __align__(16) uint8_t smem[];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int r = blockIdx.y;
-  const int n_begin = blockIdx.x * a.chunk, n_end = min(a.L, n_begin + a.chunk);
-  const int NT = (n_end - n_begin + 127) >> 7;
-  const uint32_t sb = smem_u32(smem);
-  const uint32_t bar0 = sb + K::oBAR;
-#define BAR(i) (bar0 + 8u * (uint32_t)(i))
-  volatile uint32_t* tslot = reinterpret_cast<volatile uint32_t*>(smem + K::oBAR + K::NBAR * 8);
-  volatile int* smax = reinterpret_cast<volatile int*>(smem + K::oBAR + K::NBAR * 8 + 8);
-  volatile uint32_t* wdbg = reinterpret_cast<volatile uint32_t*>(smem + K::oBAR + K::NBAR * 8 + 32);
-  if (tid < 32) wdbg[tid] = 0;
-  const float sqrtC = sqrtf((float)C);
-
-  if (tid == 0) {
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(BAR(kS + i), 1); mbar_init(BAR(kLD + i), 16); mbar_init(BAR(kTILE + i), 16); mbar_init(BAR(kTFREE + i), 8);
-    }
-    for (int i = 0; i < K::NSTG; ++i) { mbar_init(BAR(kFULL + i), 4); mbar_init(BAR(kSFREE + i), 4); }
-    *smax = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 24) tmem_alloc(smem_u32(const_cast<const uint32_t*>(tslot)), 512);
-  for (int i = tid; i < (K::oKS - K::oAX) / 16; i += kThreadsK) reinterpret_cast<uint4*>(smem + K::oAX)[i] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  // per-row scale of the gradient-side operand: |dks'| = |H' xn - sd'| <= 1 with H' = 2^e H
-  float gmax = 0.f;
-#pragma unroll
-  for (int c = 0; c < C; ++c) gmax = fmaxf(gmax, fabsf(__ldg(a.g_pre + c)));
-  if (tid < kHD) {
-    const float* hp = a.hmat + ((size_t)r * kHD + tid) * K::CL;
-    float b = fabsf(a.sd[(size_t)r * kHD + tid]);
-#pragma unroll
-    for (int c = 0; c < C; ++c) b = fmaf(fabsf(hp[c]), sqrtC * gmax, b);
-    atomicMax(const_cast<int*>(smax), __float_as_int(b));
-  }
-  __syncthreads();
-  const float bound = __int_as_float(*smax);
-  int e = 0;
-  if (bound > 0.f && bound < 1e30f) { frexpf(bound, &e); e = -e; }   // bound = m 2^(-e), m in [0.5, 1): 2^e bound < 1
-  e = max(-100, min(100, e));
-  const float hscale = exp2f((float)e), unscale = exp2f(-(float)(11 + e));
-  if (tid < kHD) {
-    const int hd = tid;
-    const float m = a.msm[((size_t)r * kHD + hd) * (2 + K::CL)], s = a.msm[((size_t)r * kHD + hd) * (2 + K::CL) + 1];
-    const float cn = 11.f - (m * kLog2e + log2f(s));
-    const float sdv = -a.sd[(size_t)r * kHD + hd] * hscale;
-    const float cn_hi = __uint_as_float(f2tf(cn)), sd_hi = __uint_as_float(f2tf(sdv));
-    const uint32_t row = (hd & 7) * 16 + (hd >> 3) * K::A_SBO;
-#pragma unroll
-    for (int k = 0; k < K::CP; ++k) {
-      float wk = 0.f, hh = 0.f;
-      if (k < C) {
-        wk = a.wqkv[(size_t)(kHD + hd) * C + k] * kLog2e;
-        hh = a.hmat[((size_t)r * kHD + hd) * K::CL + k] * hscale;
-      } else if (k == C) { wk = cn_hi; hh = sd_hi; }
-      else if (k == C + 1) { wk = cn - cn_hi; hh = sdv - sd_hi; }
-      const uint32_t off = row + (k >> 2) * 128 + (k & 3) * 4;
-      *reinterpret_cast<uint32_t*>(smem + K::oBK + off) = f2tf(wk);
-      *reinterpret_cast<uint32_t*>(smem + K::oBH + off) = f2tf(hh);
-    }
-  }
-  proxy_fence();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tm = *tslot;
-
-  if (warp < 16) {
-    // ------------------------------------------------------------------------------------------ per-element math
-    const int h = warp >> 2, quad = warp & 3;
-    const uint32_t lane_addr = tm + ((uint32_t)(quad * 32) << 16);
-    const int pos = quad * 32 + lane;
-    for (int t = 0; t < NT; ++t) {
-      const int slot = t & 1, p = t & 1;
-      mbar_wait(BAR(kS + slot), (uint32_t)((t >> 1) & 1), 40, wdbg, (uint32_t)t);
-      tc_fence_after();
-      uint32_t pk[2][8], pd[2][8];
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        uint32_t kv[16], dv[16];
-        tmem_ld16(lane_addr + slot * 256 + h * 32 + half * 16, kv);
-        tmem_ld16(lane_addr + slot * 256 + 128 + h * 32 + half * 16, dv);
-        tmem_ld_wait();
-        if (half == 1) {   // every score column of this warp is in registers: the slot may take tile t + 2
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(BAR(kLD + slot));
-        }
-#pragma unroll
-        for (int i = 0; i < 16; i += 2) {
-          const float k0 = ex2f(__uint_as_float(kv[i])), k1 = ex2f(__uint_as_float(kv[i + 1]));   // ks' = 2^11 softmax_L(k)
-          float d0, d1;
-          upk2(mul2(pk2(k0, k1), pk2(__uint_as_float(dv[i]), __uint_as_float(dv[i + 1]))), d0, d1);  // dk' = ks' dks'
-          pk[half][i >> 1] = f16x2_rn(k0, k1);
-          pd[half][i >> 1] = f16x2_rn(d0, d1);
-        }
-      }
-      if (t >= 2) mbar_wait(BAR(kTFREE + p), (uint32_t)(((t >> 1) - 1) & 1), 41, wdbg, (uint32_t)t);   // tile t - 2 read
-      uint8_t* tk = smem + K::oKS + p * K::TILE;
-      uint8_t* td = smem + K::oDK + p * K::TILE;
-#pragma unroll
-      for (int g = 0; g < 4; ++g) {
-        const uint32_t off = (uint32_t)(((4 * h + g) * 128 + pos) * 16);
-        *reinterpret_cast<uint4*>(tk + off) = make_uint4(pk[g >> 1][4 * (g & 1)], pk[g >> 1][4 * (g & 1) + 1], pk[g >> 1][4 * (g & 1) + 2], pk[g >> 1][4 * (g & 1) + 3]);
-        *reinterpret_cast<uint4*>(td + off) = make_uint4(pd[g >> 1][4 * (g & 1)], pd[g >> 1][4 * (g & 1) + 1], pd[g >> 1][4 * (g & 1) + 2], pd[g >> 1][4 * (g & 1) + 3]);
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(BAR(kTILE + p));
-    }
-  } else if (warp == 24) {
-    // ------------------------------------------------------------------------------------------ score MMAs
-    constexpr uint32_t id_s = make_idesc(kFmtTF32, 128, 128, 0, 0);
-    constexpr uint32_t hiA = (K::A_SBO >> 4) | (1u << 14);
-    const uint32_t bk = desc_lo(sb + K::oBK), bh = desc_lo(sb + K::oBH);
-    for (int t = 0; t < NT; ++t) {
-      const int slot = t & 1, st = t % K::NSTG;
-      mbar_wait(BAR(kFULL + st), (uint32_t)((t / K::NSTG) & 1), 50, wdbg, (uint32_t)t);
-      if (t >= 2) mbar_wait(BAR(kLD + slot), (uint32_t)(((t >> 1) - 1) & 1), 51, wdbg, (uint32_t)t);
-      tc_fence_after();
-      if (elect_one()) {
-        const uint32_t ax = desc_lo(sb + K::oAX + st * K::A_BYTES);
-#pragma unroll
-        for (int ks = 0; ks < K::KS; ++ks) mma_ss_tf32(tm + slot * 256, mk_desc(ax + ks * 16, hiA), mk_desc(bk + ks * 16, hiA), id_s, ks > 0);
-#pragma unroll
-        for (int ks = 0; ks < K::KS; ++ks) mma_ss_tf32(tm + slot * 256 + 128, mk_desc(ax + ks * 16, hiA), mk_desc(bh + ks * 16, hiA), id_s, ks > 0);
-        umma_commit(BAR(kS + slot));
-      }
-      __syncwarp();
-    }
-  } else if (warp < 20) {
-    // ------------------------------------------------------------------------------------------ staging
-    const int w = warp - 16, j = w * 32 + lane;
-    float gp[C];
-#pragma unroll
-    for (int c = 0; c < C; ++c) gp[c] = __ldg(a.g_pre + c);
-    float xv[C];
-    auto load_tile = [&](int t) {
-      const int n = n_begin + t * 128 + j;
-      const bool ok = n < n_end;
-#pragma unroll
-      for (int c = 0; c < C; ++c) xv[c] = ok ? __ldg(a.x + ((size_t)r * C + c) * a.L + n) : 0.f;
-    };
-    auto stage = [&](int t) {
-      const int st = t % K::NSTG;
-      const bool ok = n_begin + t * 128 + j < n_end;
-      float s2 = 0.f;
-#pragma unroll
-      for (int c = 0; c < C; ++c) s2 = fmaf(xv[c], xv[c], s2);
-      const float inv = 1.f / fmaxf(sqrtf(s2), 1e-12f);
-      float row[K::CP];
-#pragma unroll
-      for (int k = 0; k < K::CP; ++k) {
-        float v = 0.f;
-        if (k < C) v = xv[k < C ? k : 0] * (inv * sqrtC) * gp[k < C ? k : 0];
-        else if (k < C + 2) v = ok ? 1.f : 0.f;
-        row[k] = v;
-      }
-      const uint32_t arow = (uint32_t)((j & 7) * 16 + (j >> 3) * K::A_SBO);
-#pragma unroll
-      for (int c4 = 0; c4 < K::CP / 4; ++c4)
-        *reinterpret_cast<float4*>(smem + K::oAX + st * K::A_BYTES + arow + c4 * 128) =
-            make_float4(rtf32(row[4 * c4]), rtf32(row[4 * c4 + 1]), rtf32(row[4 * c4 + 2]), rtf32(row[4 * c4 + 3]));
-#pragma unroll
-      for (int c = 0; c < C; ++c) {
-        *reinterpret_cast<__half*>(smem + K::oXT + st * K::XT_BYTES + c * K::XT_ROW + j * 2) = __float2half_rn(row[c]);
-        *reinterpret_cast<float*>(smem + K::oXS + st * K::XS_BYTES + (c * 128 + j) * 4) = xv[c];
-      }
-      *reinterpret_cast<float*>(smem + K::oINV + st * 512 + j * 4) = inv;
-      proxy_fence();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(BAR(kFULL + st));
-    };
-    for (int t = 0; t < K::NSTG && t < NT; ++t) { load_tile(t); stage(t); }
-    if (NT > K::NSTG) load_tile(K::NSTG);
-    // ... and the weight-gradient product dWk' [(head, d) x 8] += dk'^T xn of every finished tile: warp w owns the
-    // (head, d) rows [32 w, 32 w + 32) (two m16 tiles, two independent accumulator chains)
-    const int g = lane >> 2, tq = lane & 3, mi = lane >> 3, mr = lane & 7;
-    float accw[2][4];
-#pragma unroll
-    for (int m = 0; m < 2; ++m)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) accw[m][i] = 0.f;
-    for (int t = 0; t < NT; ++t) {
-      const int p = t & 1, st = t % K::NSTG;
-      mbar_wait(BAR(kTILE + p), (uint32_t)((t >> 1) & 1), 61, wdbg, (uint32_t)t);
-      {
-        const uint32_t td = sb + K::oDK + p * K::TILE;
-        const uint8_t* xt = smem + K::oXT + st * K::XT_BYTES + g * K::XT_ROW + 4 * tq;
-        const uint32_t grp = (uint32_t)(4 * w + (mi & 1));
-#pragma unroll
-        for (int ks = 0; ks < 8; ++ks) {
-          uint32_t a0[4], a1[4];
-          const uint32_t prow = (uint32_t)(16 * ks + 8 * (mi >> 1) + mr);
-          ldmatrix_x4_trans(td + (grp * 128 + prow) * 16, a0);
-          ldmatrix_x4_trans(td + ((grp + 2) * 128 + prow) * 16, a1);
-          const uint32_t b0 = *reinterpret_cast<const uint32_t*>(xt + 32 * ks), b1 = *reinterpret_cast<const uint32_t*>(xt + 32 * ks + 16);
-          mma_f16_16816(accw[0], a0, b0, b1);
-          mma_f16_16816(accw[1], a1, b0, b1);
-        }
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(BAR(kTFREE + p));
-      if (t + K::NSTG < NT) {
-        mbar_wait(BAR(kSFREE + st), (uint32_t)((t / K::NSTG) & 1), 60, wdbg, (uint32_t)t);
-        stage(t + K::NSTG);
-        if (t + K::NSTG + 1 < NT) load_tile(t + K::NSTG + 1);
-      }
-    }
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int hd = w * 32 + mt * 16 + g + 8 * (i >> 1), c = 2 * tq + (i & 1);
-        if (c < C) atomicAdd(a.dwqkv + (size_t)(kHD + hd) * C + c, accw[mt][i] * unscale);
-      }
-  } else if (warp < 24) {
-    // ------------------------------------------------------------------------------------------ small products + epilogue
-    const int rw = warp - 20, g = lane >> 2, tq = lane & 3;
-    // B fragments (k = (head, d), n = channel): Wk and H' as f16, eight k16 steps
-    uint32_t bkf[8][2], bhf[8][2];
-#pragma unroll
-    for (int ks = 0; ks < 8; ++ks)
-#pragma unroll
-      for (int i = 0; i < 2; ++i) {
-        const int hd = 16 * ks + 2 * tq + 8 * i;
-        float w0 = 0.f, w1 = 0.f, h0 = 0.f, h1 = 0.f;
-        if (g < C) {
-          w0 = a.wqkv[(size_t)(kHD + hd) * C + g];
-          w1 = a.wqkv[(size_t)(kHD + hd + 1) * C + g];
-          h0 = a.hmat[((size_t)r * kHD + hd) * K::CL + g] * hscale;
-          h1 = a.hmat[((size_t)r * kHD + hd + 1) * K::CL + g] * hscale;
-        }
-        bkf[ks][i] = f16x2_rn(w0, w1);
-        bhf[ks][i] = f16x2_rn(h0, h1);
-      }
-    float dgp[C];
-#pragma unroll
-    for (int c = 0; c < C; ++c) dgp[c] = 0.f;
-    float* pf_s = reinterpret_cast<float*>(smem + K::oPF);
-    const int mi = lane >> 3, mr = lane & 7;       // ldmatrix: this lane addresses row mr of matrix mi
-    const int jpos = rw * 32 + lane;               // epilogue: this lane's position in the tile
-    float* dxn_s = reinterpret_cast<float*>(smem + K::oDXN);
-    for (int t = 0; t < NT; ++t) {
-      const int p = t & 1, st = t % K::NSTG;
-      const int n = n_begin + t * 128 + jpos;
-      const bool ok = n < n_end;
-#pragma unroll
-      for (int c = 0; c < C; ++c) {   // epilogue inputs: in flight (cp.async, no registers) while the tile is computed
-        const size_t idx = ((size_t)r * C + c) * a.L + (ok ? n : n_end - 1);
-        cp_async4(pf_s + c * 128 + jpos, a.dxnq + idx, ok);
-        cp_async4(pf_s + (C + c) * 128 + jpos, a.dres + idx, ok);
-      }
-      asm volatile("cp.async.commit_group;" ::: "memory");
-      const uint32_t tk = sb + K::oKS + p * K::TILE, td = sb + K::oDK + p * K::TILE;
-      {   // d xn' [2 x 16 positions x 8] = dk' Wk + ks' H': four independent accumulator chains (2 m-tiles x 2 products);
-          // the k-steps 2 h, 2 h + 1 belong to head h and are consumed as soon as that head's slice is written
-        float acc[2][2][4];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) (&acc[0][0][0])[i] = 0.f;
-        const uint32_t prow = (uint32_t)(rw * 32 + 8 * (mi & 1) + mr);
-#pragma unroll
-        mbar_wait(BAR(kTILE + p), (uint32_t)((t >> 1) & 1), 70, wdbg, (uint32_t)t);
-#pragma unroll
-        for (int hh = 0; hh < 4; ++hh) {
-#pragma unroll
-          for (int k2 = 0; k2 < 2; ++k2) {
-            const int ks = 2 * hh + k2;
-            const uint32_t off0 = ((uint32_t)(2 * ks + (mi >> 1)) * 128 + prow) * 16, off1 = off0 + 16 * 16;
-            uint32_t a0[4], a1[4], a2[4], a3[4];
-            ldmatrix_x4(td + off0, a0);
-            ldmatrix_x4(tk + off0, a1);
-            ldmatrix_x4(td + off1, a2);
-            ldmatrix_x4(tk + off1, a3);
-            mma_f16_16816(acc[0][0], a0, bkf[ks][0], bkf[ks][1]);
-            mma_f16_16816(acc[0][1], a1, bhf[ks][0], bhf[ks][1]);
-            mma_f16_16816(acc[1][0], a2, bkf[ks][0], bkf[ks][1]);
-            mma_f16_16816(acc[1][1], a3, bhf[ks][0], bhf[ks][1]);
-          }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(BAR(kTFREE + p));
-#pragma unroll
-        for (int mt = 0; mt < 2; ++mt) {
-          float* o = dxn_s + (rw * 32 + mt * 16 + g) * 8 + 2 * tq;
-          *reinterpret_cast<float2*>(o) = make_float2(acc[mt][0][0] + acc[mt][1][0], acc[mt][0][1] + acc[mt][1][1]);
-          *reinterpret_cast<float2*>(o + 64) = make_float2(acc[mt][0][2] + acc[mt][1][2], acc[mt][0][3] + acc[mt][1][3]);
-        }
-      }
-      __syncwarp();
-      {  // RMSNorm_pre backward + residual gradient for position jpos
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        const float inv = *reinterpret_cast<const float*>(smem + K::oINV + st * 512 + jpos * 4);
-        float uh[C], duh[C], dot = 0.f;
-#pragma unroll
-        for (int c = 0; c < C; ++c) {
-          const float xc = *reinterpret_cast<const float*>(smem + K::oXS + st * K::XS_BYTES + (c * 128 + jpos) * 4);
-          const float dxn = ok ? fmaf(dxn_s[jpos * 8 + c], unscale, pf_s[c * 128 + jpos]) : 0.f;
-          uh[c] = xc * inv;
-          dgp[c] = fmaf(dxn * uh[c], sqrtC, dgp[c]);
-          duh[c] = dxn * __ldg(a.g_pre + c) * sqrtC;
-          dot = fmaf(duh[c], uh[c], dot);
-        }
-        if (ok) {
-          const bool big = inv < 1e12f;
-#pragma unroll
-          for (int c = 0; c < C; ++c)
-            a.dx[((size_t)r * C + c) * a.L + n] = pf_s[(C + c) * 128 + jpos] + (big ? (duh[c] - uh[c] * dot) * inv : duh[c] * inv);
-        }
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(BAR(kSFREE + st));
-    }
-#pragma unroll
-    for (int c = 0; c < C; ++c) {
-      const float s1 = warp_sum(dgp[c]);
-      if (lane == 0) atomicAdd(a.dg_pre + c, s1);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 24) tmem_dealloc(tm, 512);
-#undef BAR
-}
-
-template <int C>
-static int launch_bwd_kv(const LAArgs& a, cudaStream_t st) {
-  using K = BK<C>;
-  auto kern = la_bwd_kv_tc_kernel<C>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM);
-  if (e != cudaSuccess) return (int)e;
-  dim3 grid((unsigned)a.nchunk, (unsigned)a.R);
-  kern<<<grid, kThreadsK, K::SMEM, st>>>(a);
-  DQ_LAUNCH_CHECK();
-  return 0;
-}
-
 }  // namespace tc
 
 }  // namespace dq
@@ -854,20 +472,11 @@ DQ_API int dq_la_tc_last_error(unsigned int* out6) {
 }
 namespace dq {
 
-int la_bwd_kv_tc(const LAArgs& a, int C, cudaStream_t st) {
-  switch (C) {
-    case 4: return tc::launch_bwd_kv<4>(a, st);
-    case 8: return tc::launch_bwd_kv<8>(a, st);
-    default: return -3;
-  }
-}
-
 int la_bwd_q_tc(const LAArgs& a, int C, cudaStream_t st) {
   switch (C) {
     case 4: return tc::launch_bwd_q<4>(a, st);
     case 8: return tc::launch_bwd_q<8>(a, st);
     case 12: return tc::launch_bwd_q<12>(a, st);
-    case 16: return tc::launch_bwd_q<16>(a, st);
     default: return -3;
   }
 }

@@ -59,14 +59,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, uint32_
   if (dbg) dbg[threadIdx.x >> 5] = 0;
 }
 
-__device__ __forceinline__ uint64_t umma_desc_ns(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)((sbo >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;   // descriptor version (sm_100)
-  return d;
-}
 // low / high words of a no-swizzle descriptor (LBO = 128 B everywhere in these kernels); advancing the start address by
 // b bytes adds b >> 4 to the low word
 __device__ __forceinline__ uint32_t desc_lo(uint32_t saddr) { return ((saddr >> 4) & 0x3FFF) | ((128u >> 4) << 16); }
@@ -197,36 +189,6 @@ __device__ __forceinline__ uint32_t bf16x2_rn(float lo, float hi) {
   uint32_t r;
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r;
-}
-// f16x2 {lo, hi}, round to nearest (lo in the low half = lower element index)
-__device__ __forceinline__ uint32_t f16x2_rn(float lo, float hi) {
-  uint32_t r;
-  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-  return r;
-}
-// ---- warp-level tensor-core path for the SMALL products (N = 8 channels): a tcgen05.mma costs 76-119 cycles whatever N is,
-// an m16n8k16 mma.sync a handful - products with 8-16 output columns belong here
-// four 8x8 b16 matrices; lane l supplies the address of row (l % 8) of matrix (l / 8)
-__device__ __forceinline__ void ldmatrix_x4(uint32_t saddr, uint32_t (&r)[4]) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(saddr));
-}
-__device__ __forceinline__ void ldmatrix_x4_trans(uint32_t saddr, uint32_t (&r)[4]) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(saddr));
-}
-// D (16 x 8, fp32) += A (16 x 16, f16) B (16 x 8, f16)
-__device__ __forceinline__ void mma_f16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-// 4-byte cp.async (zero fill when !ok): global -> shared without registers (a register prefetch gets spilled: the spill
-// store then waits for the load)
-__device__ __forceinline__ void cp_async4(float* dst_smem, const float* src, bool ok) {
-  const uint32_t d = smem_u32(dst_smem);
-  const int sz = ok ? 4 : 0;
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(d), "l"(src), "r"(sz) : "memory");
 }
 // The TF32 MMA truncates the low 13 mantissa bits of an fp32 operand; adding half an ulp first makes it round to nearest.
 __device__ __forceinline__ float rtf32(float x) { return __uint_as_float(__float_as_uint(x) + 0x1000u); }
