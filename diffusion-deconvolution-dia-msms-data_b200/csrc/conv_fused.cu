@@ -1282,8 +1282,12 @@ static int launch_fused(ConvBwdFusedArgs a, cudaStream_t st) {
 template <int K>
 static int dispatch_fused(const ConvBwdFusedArgs& a, int cout, cudaStream_t st) {
   const bool v4 = (a.L % 4 == 0);
-  // 16-byte aligned rows: bulk-async-copy pipeline
+  // 16-byte aligned rows of the staged inputs: bulk-async-copy pipeline
   const bool al = v4 && ((((size_t)a.dy | (size_t)a.x1 | (size_t)a.u | (size_t)a.x2) & 15) == 0);
+  // the FFMA variants (bulk pipeline with NCI == 0, and conv_bwd_fused_kernel with VEC = 4) also read dadd / the old dx
+  // and store dx with float4 / float2 accesses; the tensor-core variants store dx scalar and check each dadd / old-dx row
+  // before their 16-byte copies, so only `al` applies to them (a null pointer is 0: it never vetoes)
+  const bool alv = al && ((((size_t)a.dadd | (size_t)a.dx1 | (size_t)a.dx2) & 15) == 0);
   // the pipelined kernel covers: plain conv, or RMSNorm (+ scale/shift) + SiLU epilogue; channel counts in fours
   const bool epi_ok = !a.u || (a.g && a.act == 1);
   const int cin = a.c1 + a.c2;
@@ -1309,11 +1313,11 @@ static int dispatch_fused(const ConvBwdFusedArgs& a, int cout, cudaStream_t st) 
       if (a.L >= 128 && a.u && a.g && a.act == 1 && ch4 && !a.dadd) {
         const int nci = (cin + 7) / 8;
         if (al2) {
-          if (cout == 4) return launch_fused_tma<4, 3, 4, 128, true, true, true>(a, st);
+          if (cout == 4 && alv) return launch_fused_tma<4, 3, 4, 128, true, true, true>(a, st);
           if (cout == 8) {
             if (nci == 1) return launch_fused_tma<8, 3, 2, 128, true, true, true, 1>(a, st);
             if (nci == 2) return launch_fused_tma<8, 3, 2, 128, true, true, true, 2>(a, st);
-            return launch_fused_tma<8, 3, 2, 128, true, true, true>(a, st);
+            if (alv) return launch_fused_tma<8, 3, 2, 128, true, true, true>(a, st);
           }
           if (cout == 12 && nci == 3) return launch_fused_tma<12, 3, 1, 128, true, true, true, 3>(a, st);
           if (cout == 16 && nci == 4) return launch_fused_tma<16, 3, 1, 128, true, true, true, 4>(a, st);
@@ -1326,7 +1330,7 @@ static int dispatch_fused(const ConvBwdFusedArgs& a, int cout, cudaStream_t st) 
     return 1;    // not covered: the caller runs the two convolutions separately
   }
   if (a.L >= 128 && epi_ok && ch4) {
-    if (al) {
+    if (alv) {
       switch (cout) {
         case 4: return launch_fused_tma_epi<4, K, 4, 128, true>(a, st);
         case 8: return launch_fused_tma_epi<8, K, 2, 128, true>(a, st);
@@ -1344,10 +1348,11 @@ static int dispatch_fused(const ConvBwdFusedArgs& a, int cout, cudaStream_t st) 
       }
     }
   }
+  // VEC = 4 reads dy / u / x1 / x2 / dadd / the old dx and stores dx as float4: every one of them must be 16-byte aligned
   switch (cout) {
-    case 1: return v4 ? launch_fused<1, K, 4, 4>(a, st) : launch_fused<1, K, 4, 1>(a, st);
-    case 4: return v4 ? launch_fused<4, K, 4, 4>(a, st) : launch_fused<4, K, 4, 1>(a, st);
-    case 8: return v4 ? launch_fused<8, K, 4, 4>(a, st) : launch_fused<8, K, 4, 1>(a, st);
+    case 1: return alv ? launch_fused<1, K, 4, 4>(a, st) : launch_fused<1, K, 4, 1>(a, st);
+    case 4: return alv ? launch_fused<4, K, 4, 4>(a, st) : launch_fused<4, K, 4, 1>(a, st);
+    case 8: return alv ? launch_fused<8, K, 4, 4>(a, st) : launch_fused<8, K, 4, 1>(a, st);
     case 12: return launch_fused<12, K, 2, 1>(a, st);
     case 16: return launch_fused<16, K, 2, 1>(a, st);
     case 24: return launch_fused<24, K, 1, 1>(a, st);

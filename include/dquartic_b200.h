@@ -57,6 +57,11 @@ int dq_mse(const float* eps, const float* noise, double* loss_sum, float* deps, 
 int dq_add_inplace(float* a, const float* b, long n, void* stream);
 
 /* ---- down/up path (model/unet1d.py) ------------------------------------------------------------------- */
+/* Alignment: the tensor pointers of dq_conv1d_fwd, dq_resblock_fwd, dq_block_bwd, dq_conv1d_bwd_data/_weight,
+ * dq_conv_bwd_fused, dq_conv_bwd_fused_res, dq_upconv_bwd_fused, dq_downconv_bwd_fused and dq_initconv_bwd need only
+ * 4-byte alignment (a view that starts at any float of an allocation is accepted).  Their 16-byte vector / bulk-copy
+ * paths are taken only when every pointer such a path touches is 16-byte aligned and the row length allows it; otherwise
+ * a 4-byte path runs (or the call returns 1 and the documented composition applies). */
 /* Fused Conv1d (+concat of two sources, ConditionalScaleShift on source 1, bias, RMSNorm, scale/shift, act,
  * residual): Block.forward 248-268, ResnetBlock 302-323, init_conv 1107-1117, Downsample 110, Upsample 93-96,
  * skip cats 1151/1154/1160, final_conv 1163, attn_cond_proj 976-978. */

@@ -17,23 +17,23 @@ COVERED_BY = {
     "dq_scale_by": "test_model_gpu.py::test_train_step_loss_and_gradients_match_reference_golden",
     "dq_add_inplace": "test_model_gpu.py::test_train_step_loss_and_gradients_match_reference_golden",
     "dq_ncl_nlc": "test_model_gpu.py::test_train_step_loss_and_gradients_match_reference_golden",
-    "dq_block_bwd": "test_model_gpu.py::test_train_step_loss_and_gradients_match_reference_golden",
+    "dq_block_bwd": "test_updown_convs_gpu.py::test_attn_cond_proj_convs_and_gelu_block_backward_over_rt",
     "dq_add_mul": "test_model_gpu.py::test_ddim_sampling_matches_reference_golden",
     "dq_ddim_step_x0": "test_round2_gpu.py::test_secondary_modes_vs_oracle",
     "dq_cosine_sums": "test_round2_gpu.py::test_predict_returns_reference_dicts_and_predict_batch_scores_every_window",
     "dq_map_scores": "test_validation_gpu.py::test_map_scores_match_the_float64_oracle",
-    "dq_initconv_bwd": "test_round2_gpu.py::test_initconv_one_pass_backward_matches_generic_path",
+    "dq_initconv_bwd": "test_updown_convs_gpu.py::test_init_conv_forward_and_one_pass_backward_per_element",
     "dq_sample_dot": "test_round2_gpu.py::test_initconv_one_pass_backward_matches_generic_path",
-    "dq_conv1d_fwd": "test_kernels_gpu.py::test_resample_convs",
+    "dq_conv1d_fwd": "test_updown_convs_gpu.py::test_resampling_and_plain_conv_per_element_at_training_shape",
     "dq_conv1d_bwd_data": "test_kernels_gpu.py::test_resample_convs",
-    "dq_conv1d_bwd_weight": "test_kernels_gpu.py::test_resample_convs",
-    "dq_resblock_fwd": "test_kernels_gpu.py::test_resnet_block_fwd_bwd",
-    "dq_conv_bwd_fused": "test_kernels_gpu.py::test_resnet_block_fwd_bwd",
-    "dq_conv_bwd_fused_res": "test_kernels_gpu.py::test_resnet_block_fwd_bwd",
-    "dq_upconv_bwd_fused": "test_round2_gpu.py::test_upsample_backward_one_pass_matches_three_pass_composition",
+    "dq_conv1d_bwd_weight": "test_updown_convs_gpu.py::test_attn_cond_proj_convs_and_gelu_block_backward_over_rt",
+    "dq_resblock_fwd": "test_updown_convs_gpu.py::test_resnet_block_per_element_at_training_shape",
+    "dq_conv_bwd_fused": "test_updown_convs_gpu.py::test_resnet_block_per_element_at_training_shape",
+    "dq_conv_bwd_fused_res": "test_updown_convs_gpu.py::test_resnet_block_per_element_at_training_shape",
+    "dq_upconv_bwd_fused": "test_updown_convs_gpu.py::test_resampling_and_plain_conv_per_element_at_training_shape",
     "dq_upsample2x": "test_round2_gpu.py::test_upsample_backward_one_pass_matches_three_pass_composition",
     "dq_fold2x": "test_round2_gpu.py::test_upsample_backward_one_pass_matches_three_pass_composition",
-    "dq_downconv_bwd_fused": "test_round2_gpu.py::test_downsample_backward_one_pass_matches_reindexing_composition",
+    "dq_downconv_bwd_fused": "test_updown_convs_gpu.py::test_resampling_and_plain_conv_per_element_at_training_shape",
     "dq_s2d": "test_round2_gpu.py::test_downsample_backward_one_pass_matches_reindexing_composition",
     "dq_d2s": "test_round2_gpu.py::test_downsample_backward_one_pass_matches_reindexing_composition",
     "dq_down_w": "test_round2_gpu.py::test_downsample_backward_one_pass_matches_reindexing_composition",

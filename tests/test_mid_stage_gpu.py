@@ -10,37 +10,17 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from _util import TINY, make_net
+from _util import NAN, TINY, U, _act_bounds, _act_ref, _check, _exp_ulp, _nan, _nan_empty, _restore_empty, make_net
 
 pytestmark = pytest.mark.gpu
 
-U = 2.0 ** -24          # fp32 unit roundoff
 UB = 2.0 ** -8          # bf16 unit roundoff (round to nearest)
 GEMM_REL = 1e-5         # |C - R| <= 1e-5 * (|A| . |B|^T + |bias| + |C_old|)
 HD, HEADS = 128, 4
-NAN = float("nan")
 BIG = dict(TINY, downsample_dim=40000)   # mid channels 16 * 625 = 10000
 
 
 # ---------------------------------------------------------------------------------------------- helpers
-def _nan(*shape, dtype=torch.float32):
-    return torch.full(shape, NAN, dtype=dtype, device="cuda")
-
-
-def _check(tag, got, ref, bound):
-    """Every element within its bound (a NaN fails).  Prints the worst error / bound."""
-    err = (got.double() - ref).abs()
-    ok = err <= bound
-    if not bool(ok.all()):
-        bad = (~ok).nonzero()
-        i = tuple(bad[0].tolist())
-        raise AssertionError(f"{tag}: {bad.shape[0]} of {ok.numel()} elements out of bound; first {i}: "
-                             f"got {float(got[i])}, ref {float(ref[i])}, bound {float(bound[i])}")
-    frac = float((err / bound.clamp_min(1e-300)).max())
-    print(f"BOUND {tag}: max err / bound = {frac:.3g}")
-    return frac
-
-
 def _shift(A, o):
     """A_tap[m] = A[m + o], zero outside (TMA's out-of-range fill)."""
     if o == 0:
@@ -71,17 +51,6 @@ def _pick_bn(m_tiles, N, nz, sms):
 def _report_bn(tag, M, N, nz=1):
     sms = torch.cuda.get_device_properties(0).multi_processor_count
     print(f"PICK_BN {tag}: M={M} N={N} nz={nz} -> bn {_pick_bn((M + 127) // 128, N, nz, sms)}")
-
-
-def _nan_empty(net):
-    """Make net._empty return NaN-filled tensors (an element a kernel should write but does not stays NaN)."""
-    def empty(*shape, dtype=torch.float32):
-        return torch.full(shape, NAN, dtype=dtype, device=net._flat.device)
-    net._empty = empty
-
-
-def _restore_empty(net):
-    net.__dict__.pop("_empty", None)
 
 
 @pytest.fixture(scope="module")
@@ -300,11 +269,6 @@ def test_gemm_mid_attention_shapes(big, kind):
 
 
 # ---------------------------------------------------------------------------------------------- 2. fp32 kernels
-def _exp_ulp(x):
-    """CUDA Programming Guide, intrinsic functions: __expf(x) has a maximum error of 2 + floor(|1.173 x|) ulp."""
-    return 2 + torch.floor((1.173 * x).abs())
-
-
 # (ss, act, upad, dhpad, opad, du mode): du mode "bf16" = padded/plain bf16 output, "f32" = fp32 output,
 # "f32acc" = accumulate into fp32, "both" = fp32 + bf16.  dg, dbias and (with ss) dss are always accumulated.
 ROWNORM_CASES = [
@@ -633,42 +597,6 @@ def test_time_embed_against_float64(tiny, dim):
     R = torch.cat((a.sin(), a.cos()), dim=1)
     ba = U * a.abs() * (4 + (kf * neg_e).abs())[None]
     _check(f"time_embed dim={dim}", out, R, torch.cat((ba, ba), dim=1) * 2 + 4 * U)
-
-
-def _act_ref(z, act):
-    if act == 1:
-        return z * torch.sigmoid(z), torch.sigmoid(z) * (1 + z * (1 - torch.sigmoid(z)))
-    if act == 2:
-        cdf = 0.5 * (1 + torch.erf(z / math.sqrt(2)))
-        return z * cdf, cdf + z * torch.exp(-0.5 * z * z) / math.sqrt(2 * math.pi)
-    if act == 3:
-        sp = torch.where(z > 20, z, torch.log1p(torch.exp(z)))
-        return sp, torch.where(z > 20, torch.ones_like(z), torch.sigmoid(z))
-    return z, torch.ones_like(z)
-
-
-def _act_bounds(z, act):
-    """Per-element absolute error bounds of the kernel's fp32 act_fwd / act_bwd (csrc/common.cuh).
-    SiLU and the GELU derivative use __expf, whose error the CUDA Programming Guide bounds by 2 + floor(|1.173 x|) ulp;
-    expf, erff and log1pf are within 2 ulp."""
-    za = z.abs()
-    if act == 1:
-        e1 = U * (_exp_ulp(z) + 4)
-        s = torch.sigmoid(z)
-        return 2 * e1 * (z * s).abs(), 2 * (e1 + 4 * U) * s * (1 + za * (1 + s))
-    if act == 2:
-        erf = torch.erf(z / math.sqrt(2)).abs()
-        pdf = torch.exp(-0.5 * z * z) / math.sqrt(2 * math.pi)
-        fwd = 6 * U * 0.5 * za * (1 + erf)
-        e2 = U * (_exp_ulp(0.5 * z * z) + z * z + 4)
-        return fwd, 2 * (4 * U * (1 + erf) + za * pdf * e2)
-    if act == 3:
-        E = torch.exp(torch.clamp(z, max=20))
-        sp, dsp = _act_ref(z, 3)
-        small = z <= 20
-        fwd = torch.where(small, U * (4 * E / (1 + E) + 3 * sp.abs()), torch.zeros_like(z))
-        return fwd, torch.where(small, 6 * U * dsp.abs(), torch.zeros_like(z))
-    return torch.zeros_like(z), torch.zeros_like(z)
 
 
 @pytest.mark.parametrize("act", [0, 1, 2, 3])

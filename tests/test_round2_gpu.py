@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 import torch
 
-from _util import TINY, make_net, rel_err
+from _util import TINY, _misaligned, make_net, rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -405,15 +405,6 @@ def test_init_conv_forward_pipelined_kernel_vs_torch(L, rt):
     ref = torch.nn.functional.conv1d(torch.cat([cond * sc + sh, x], 1), net._w("init_conv.weight").view(cout, 2, 7),
                                      net._w("init_conv.bias"), padding=3)
     assert rel_err(y, ref) < 1e-5, rel_err(y, ref)
-
-
-def _misaligned(t):
-    """A contiguous copy of `t` whose base address is 4 bytes past a 16-byte boundary (kernels must leave their vector paths)."""
-    flat = torch.empty(t.numel() + 1, dtype=t.dtype, device=t.device)
-    v = flat[1:].view(t.shape)
-    v.copy_(t)
-    assert v.is_contiguous() and v.data_ptr() % 16 == 4
-    return v
 
 
 def test_resampling_kernels_accept_tensors_that_are_not_16_byte_aligned():
